@@ -6,6 +6,7 @@
   python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
          bench.py --gpus N --steps K --warmup W               # N ranks, one per GPU, NCCL all-gather of records
   python bench.py --impl reference --steps 3 --warmup 3       # the reference path's CPU restatement (oracle)
+  python bench.py --steps 20 --warmup 5 --dump-outputs DIR     # also write the last timed step's outputs to DIR/<name>.npy
 
 Prints ONE JSON line (contract in the task statement): value = whole-job images/s with inputs resident in HBM,
 e2e = same metric through the public API with pinned-host inputs (H2D and D2H inside the timed region),
@@ -266,6 +267,7 @@ def run_ours(a):
 
     c4 = a.mode == 'c4'                                            # BASELINE configs[3]: CamCalib bypassed, dataset-supplied (R, K)
     B = a.batch if a.batch > 0 else (128 if c4 else 256)           # per-GPU batch (weak scaling)
+    torch.manual_seed(0)                                           # the heads' constructor initialisation: same weights every run
     cc = sb.CameraRegressorNetwork('resnet50')
     randomize_module_(cc.backbone, 1)
     hmr = sb.HMR(a.backbone, use_cam=True, use_cam_feats=True, smpl_data=synthetic_smpl_data(0), mean_params=synthetic_mean_params(0))
@@ -342,14 +344,15 @@ def run_ours(a):
         host_ms = []
         for i in range(steps):
             host_ms.append((time.perf_counter() - t_host0) * 1e3)  # when the launching thread STARTED enqueuing step i
-            fn()
+            last = fn()
             marks[i].record()
             if mid is not None and i % 64 == min(steps // 2, 32):
                 mid()                                              # wakes the NVML helper thread; never blocks this thread
         if gatherer is not None:
-            gatherer.flush()                                       # the last gather completes inside the timed region
+            last = gatherer.flush()                                # the last gather completes inside the timed region
         e1.record()
         torch.cuda.synchronize(dev)
+        timed.last = last.cpu() if a.dump_outputs else None       # the buffer is reused by later calls: copy it out now
         if world > 1:
             dist.barrier()
         ms = torch.tensor([e0.elapsed_time(e1)], device=dev)
@@ -382,6 +385,8 @@ def run_ours(a):
         dist.all_gather_object(spreads, step_spread)
         step_spread['per_rank'] = spreads
     clocks = sampler.stop() if rank == 0 else None
+    if a.dump_outputs and rank == 0:
+        dump_outputs(a.dump_outputs, timed.last, [k for k in c4_out] if c4 else None)
     ms_per_step = total_ms / a.steps
     value = world * B * a.steps / (total_ms * 1e-3)
     launches_per_step = hmr.last_launches() if c4 else pipe.launches_per_step()
@@ -537,6 +542,25 @@ def run_ours(a):
     return out
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, record, keys=None):
+    """Writes the per-image arrays a caller of the timed path receives from its last step (``unpack_record`` of the packed
+    records, every rank's rows after the all-gather) as ``out_dir/<name>.npy``, float32.  Above DUMP_LIMIT_BYTES in all, a
+    fixed seeded sample of the images is written (same rows for the same arguments), so two builds can be compared."""
+    import numpy as np
+    import spec_b200 as sb
+    n = record.shape[0]
+    keep = max(1, min(n, DUMP_LIMIT_BYTES // (record.shape[1] * 4)))
+    if keep < n:
+        record = record[torch.from_numpy(np.sort(np.random.RandomState(0).choice(n, keep, replace=False)))]
+    os.makedirs(out_dir, exist_ok=True)
+    for k, v in sb.unpack_record(record).items():
+        if keys is None or k in keys:
+            np.save(os.path.join(out_dir, f'{k}.npy'), v.numpy().astype(np.float32))
+
+
 _JSON_FD = None
 
 
@@ -577,7 +601,13 @@ def main():
     ap.add_argument('--no-cpu-baseline', action='store_true')
     ap.add_argument('--profile-range', action='store_true', help='only run the steps inside cudaProfilerStart/Stop (for ncu --profile-from-start off)')
     ap.add_argument('--cpu-sample', type=int, default=16, help='images per CPU-oracle step (bounded sample)')
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help="write the last timed step's outputs as DIR/<name>.npy (float32, at most 64 MB: a fixed sample of the images beyond that)")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error('--steps must be at least 1')
+    if a.dump_outputs and a.impl != 'ours':
+        ap.error('--dump-outputs writes the outputs of --impl ours')
     if a.warmup < 3:
         a.warmup = 3
     if a.impl == 'reference':

@@ -20,8 +20,8 @@ The reference keeps the arithmetic of this path in two un-vendored third-party p
   spec/models/hmr.py:28-122 (HMR), camcalib/cam_utils.py:39-63,110-145 (soft-argmax decode, bin tables) and
   spec/utils/cam_params.py:24-50 (pkl hand-off, R / K assembly) -- are EXECUTED UNMODIFIED from /root/reference with ``pare``
   stubbed in sys.modules by this package's restatements (tests/golden/reference_wrappers.py).  oracle/models.py and
-  oracle/geometry.py agree with them BIT FOR BIT on three configurations (tests/test_reference_wrappers.py, live when the
-  reference is mounted), and the outputs of that reference run are committed as tests/golden/reference_wrappers.npz, which
+  oracle/geometry.py agree with them BIT FOR BIT on three configurations (checked whenever tests/golden/reference_wrappers.py regenerates
+  the fixtures), and the outputs of that reference run are committed as tests/golden/reference_wrappers.npz, which
   the oracle (CPU test) and the CUDA path (tests/test_gpu_parity.py::test_against_reference_wrapper_fixture) are compared
   with everywhere.  That run surfaced one real discrepancy, fixed in geometry.cam_params_from_angles: the demo computes
   f_pix in NumPy float64 (NumPy-1.x promotion) before it is stored in the float32 K;

@@ -119,7 +119,7 @@ def cam_params_from_angles(vfov, pitch, roll, img_h, img_w):
     img_w = torch.as_tensor(img_w, dtype=torch.float32).expand(B) if not torch.is_tensor(img_w) else img_w.float()
     # scripts/camcalib_demo.py:127 computes this in NumPy from a float32 0-d array and Python floats: float64 under the
     # NumPy 1.x promotion rules the reference pins; read_cam_params then stores it into a float32 tensor (cam_params.py:43).
-    # Checked bit for bit against the unmodified reference code in tests/test_reference_wrappers.py.
+    # Checked bit for bit against the unmodified reference code by tests/golden/reference_wrappers.py.
     f_pix = (img_h.double() / 2. / torch.tan(vfov.double() / 2.)).float()
     eul = torch.stack([pitch, torch.zeros_like(pitch), roll], 1).float()
     R = batch_euler2matrix(eul)

@@ -1,19 +1,21 @@
-"""Runs the UNMODIFIED reference wrapper code of the hot path -- /root/reference/camcalib/model.py (CameraRegressorNetwork),
-spec/models/hmr.py (HMR), camcalib/cam_utils.py (convert_preds_to_angles) and spec/utils/cam_params.py (read_cam_params) --
-in this container, and writes what it produced to tests/golden/reference_wrappers.npz.
+"""Runs the UNMODIFIED reference wrapper code of the hot path -- camcalib/model.py (CameraRegressorNetwork),
+spec/models/hmr.py (HMR), camcalib/cam_utils.py (convert_preds_to_angles) and spec/utils/cam_params.py (read_cam_params) of a
+checkout of the original SPEC repository -- and writes what it produced to tests/golden/reference_wrappers.npz and
+tests/golden/reference_wrappers_alt_seeds.npz, plus the reference's own name tables, soft-argmax bin ranges and public
+signatures to tests/golden/reference_tables.json.
 
 Those four files import the un-vendored ``pare`` package (requirements.txt:28, no commit pinned; not installable offline).
 ``install_pare_stubs`` puts stand-ins for exactly the names they import into ``sys.modules`` -- backed by the oracle's
 restatements of the pare / smplx internals (oracle/resnet.py, hrnet.py, head.py, geometry.py) -- and ``load_reference`` then
 executes the reference files from where they lie (importlib, by path; nothing is copied).  So everything that IS in
-/root/reference for this path -- constructor wiring, the eval()-by-name backbone selection, the forward glue, the cam_vfov
+the reference for this path -- constructor wiring, the eval()-by-name backbone selection, the forward glue, the cam_vfov
 formula, the soft-argmax bin ranges built from scipy/np.linspace, the pkl hand-off and K assembly -- is the reference's own
-code producing the fixture; what stays recalled is pare's / smplx's internals behind the stubs (oracle/__init__.py).
+code producing the fixtures; what stays recalled is pare's / smplx's internals behind the stubs (oracle/__init__.py).
 
-    python -m tests.golden.reference_wrappers          # regenerate the fixture (needs /root/reference)
+    python -m tests.golden.reference_wrappers <path to a SPEC checkout>          # regenerate the fixtures
 
-tests/test_reference_wrappers.py compares oracle/models.py + oracle/geometry.py with the live reference wrappers when the
-reference is mounted and with the committed fixture everywhere (the GPU box has no /root/reference).
+tests/test_reference_wrappers.py, tests/test_oracle.py and tests/test_boundary.py compare oracle/models.py, oracle/geometry.py,
+oracle/constants.py and the product's signatures with these committed fixtures; the tests never read the reference itself.
 """
 import importlib.util
 import os
@@ -27,15 +29,13 @@ ROOT = os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__)
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
 
-REF = '/root/reference'
-FIXTURE = os.path.join(os.path.dirname(os.path.abspath(__file__)), 'reference_wrappers.npz')
+GOLDEN = os.path.dirname(os.path.abspath(__file__))
+FIXTURE = os.path.join(GOLDEN, 'reference_wrappers.npz')
+ALT_FIXTURE = os.path.join(GOLDEN, 'reference_wrappers_alt_seeds.npz')
+TABLES = os.path.join(GOLDEN, 'reference_tables.json')
 _STUB_NAMES = ['pare', 'pare.models', 'pare.models.backbone', 'pare.models.backbone.utils', 'pare.models.backbone.hrnet',
                'pare.models.head', 'pare.models.layers', 'pare.models.layers.softargmax', 'pare.utils', 'pare.utils.geometry',
                'pare.utils.train_utils']
-
-
-def reference_available():
-    return os.path.exists(os.path.join(REF, 'spec', 'models', 'hmr.py'))
 
 
 def install_pare_stubs():
@@ -95,21 +95,21 @@ def remove_pare_stubs(saved):
             sys.modules[n] = m
 
 
-def _load_by_path(name, rel):
-    spec = importlib.util.spec_from_file_location(name, os.path.join(REF, rel))
+def _load_by_path(ref_root, name, rel):
+    spec = importlib.util.spec_from_file_location(name, os.path.join(ref_root, rel))
     mod = importlib.util.module_from_spec(spec)
     spec.loader.exec_module(mod)
     return mod
 
 
-def load_reference():
-    """Executes the four reference files (unmodified, from /root/reference) with the pare stubs in place."""
+def load_reference(ref_root):
+    """Executes the four reference files (unmodified, from the SPEC checkout at ``ref_root``) with the pare stubs in place."""
     saved = install_pare_stubs()
     try:
-        return {'model': _load_by_path('_specref_camcalib_model', 'camcalib/model.py'),
-                'hmr': _load_by_path('_specref_spec_models_hmr', 'spec/models/hmr.py'),
-                'cam_utils': _load_by_path('_specref_camcalib_cam_utils', 'camcalib/cam_utils.py'),
-                'cam_params': _load_by_path('_specref_spec_utils_cam_params', 'spec/utils/cam_params.py')}
+        return {'model': _load_by_path(ref_root, '_specref_camcalib_model', 'camcalib/model.py'),
+                'hmr': _load_by_path(ref_root, '_specref_spec_models_hmr', 'spec/models/hmr.py'),
+                'cam_utils': _load_by_path(ref_root, '_specref_camcalib_cam_utils', 'camcalib/cam_utils.py'),
+                'cam_params': _load_by_path(ref_root, '_specref_spec_utils_cam_params', 'spec/utils/cam_params.py')}
     finally:
         remove_pare_stubs(saved)
 
@@ -121,6 +121,16 @@ CASES = {
     'spec_hrnet_w32_conv': dict(hmr='hrnet_w32-conv', camcalib='resnet34', fc_layers=3, batch=2, size=64, use_cam=True, use_cam_feats=True),
     'hmr_resnet34_nocam': dict(hmr='resnet34', camcalib=None, fc_layers=1, batch=3, size=64, use_cam=False, use_cam_feats=False),
 }
+SEED0, ALT_SEED0 = 40, 60               # case i runs with seed SEED0 + i (FIXTURE) and ALT_SEED0 + i (ALT_FIXTURE)
+# ALT_FIXTURE keeps every output but the vertices whole; of those it keeps this fixed sample, so that it stays small
+ALT_VERTEX_IDS = np.sort(np.random.RandomState(0).choice(6890, 96, replace=False))
+
+
+def alt_sample(out):
+    """What ALT_FIXTURE stores of one case's outputs."""
+    out = dict(out)
+    out['hmr_smpl_vertices'] = out['hmr_smpl_vertices'][:, ALT_VERTEX_IDS]
+    return out
 
 
 def case_inputs(cfg, seed):
@@ -224,20 +234,60 @@ def run_oracle_case(cfg, seed):
     return out
 
 
-def main():
+def reference_tables(ref_root, ref):
+    """The reference's name tables (spec/constants.py), the end points of its soft-argmax bin tables (cam_utils.py:39,55) and
+    the argument lists of the drop-in classes' constructors and forwards (model.py:25-31; hmr.py:29-41,82-91)."""
+    import ast
+    path = os.path.join(ref_root, 'spec', 'constants.py')
+    ns = {}
+    src = open(path).read()
+    exec(compile(src.split('# Permutation of SMPL pose parameters')[0].replace('import numpy as np', ''), path, 'exec'),
+         {'np': np}, ns)
+    out = {k: ns[k] for k in ('JOINT_NAMES', 'JOINT_MAP', 'H36M_TO_J14', 'IMG_NORM_MEAN')}
+    cu = ref['cam_utils']
+    out['bins'] = {n: [float(np.min(getattr(cu, n))), float(np.max(getattr(cu, n)))] for n in ('vfov_bins', 'pitch_bins')}
+    sigs = {}
+    for rel, cls_name in (('spec/models/hmr.py', 'HMR'), ('camcalib/model.py', 'CameraRegressorNetwork')):
+        tree = ast.parse(open(os.path.join(ref_root, rel)).read())
+        cls = [n for n in tree.body if isinstance(n, ast.ClassDef) and n.name == cls_name][0]
+        for f in cls.body:
+            if isinstance(f, ast.FunctionDef) and f.name in ('__init__', 'forward'):
+                sigs[f'{cls_name}.{f.name}'] = [a.arg for a in f.args.args][1:]
+    out['signatures'] = sigs
+    return out
+
+
+def main(ref_root, out_dir=GOLDEN):
+    import json
     import tempfile
-    if not reference_available():
-        raise SystemExit('/root/reference is not mounted: the fixture can only be regenerated in the build container')
+    if not os.path.exists(os.path.join(ref_root, 'spec', 'models', 'hmr.py')):
+        raise SystemExit(f'{ref_root} is not a checkout of the SPEC repository')
     torch.set_num_threads(4)
-    ref = load_reference()
-    blob = {}
+    ref = load_reference(ref_root)
+    blob, alt = {}, {'vertex_ids': ALT_VERTEX_IDS}
+    differ = []
     with tempfile.TemporaryDirectory() as tmp:
         for i, (name, cfg) in enumerate(CASES.items()):
-            for k, v in run_reference_case(ref, cfg, 40 + i, tmp).items():
-                blob[f'{name}/{k}'] = v
-    np.savez_compressed(FIXTURE, **blob)
-    print('wrote', FIXTURE, f'{os.path.getsize(FIXTURE) / 1e6:.2f} MB,', len(blob), 'arrays')
+            for seed, dst, keep in ((SEED0 + i, blob, lambda o: o), (ALT_SEED0 + i, alt, alt_sample)):
+                out = run_reference_case(ref, cfg, seed, tmp)
+                ora = run_oracle_case(cfg, seed)       # same process, same CPU kernels: the oracle must agree bit for bit
+                differ += [f'{name}/{k} (seed {seed})' for k in out if out[k].shape != ora[k].shape or not np.array_equal(out[k], ora[k])]
+                for k, v in keep(out).items():
+                    dst[f'{name}/{k}'] = v
+    if differ:
+        raise SystemExit('the oracle differs from the reference in ' + ', '.join(differ))
+    for path, arrays in ((FIXTURE, blob), (ALT_FIXTURE, alt)):
+        path = os.path.join(out_dir, os.path.basename(path))
+        np.savez_compressed(path, **arrays)
+        print('wrote', path, f'{os.path.getsize(path) / 1e6:.2f} MB,', len(arrays), 'arrays')
+    path = os.path.join(out_dir, os.path.basename(TABLES))
+    with open(path, 'w') as fh:
+        json.dump(reference_tables(ref_root, ref), fh, indent=1)
+        fh.write('\n')
+    print('wrote', path)
 
 
 if __name__ == '__main__':
-    main()
+    if len(sys.argv) not in (2, 3):
+        raise SystemExit('usage: python -m tests.golden.reference_wrappers <SPEC checkout> [output directory]')
+    main(*sys.argv[1:])

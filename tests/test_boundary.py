@@ -48,20 +48,15 @@ def test_signatures_match_reference():
 
 
 def test_reference_signatures_if_mounted():
-    """Parse the reference sources (dev container only) and compare argument lists literally."""
-    p = '/root/reference/spec/models/hmr.py'
-    if not os.path.exists(p):
-        pytest.skip('reference not mounted')
-    import ast
-    tree = ast.parse(open(p).read())
-    cls = [n for n in tree.body if isinstance(n, ast.ClassDef) and n.name == 'HMR'][0]
-    fns = {f.name: [a.arg for a in f.args.args] for f in cls.body if isinstance(f, ast.FunctionDef)}
-    assert fns['forward'][1:] == list(inspect.signature(sb.HMR.forward).parameters)[1:8]
-    assert fns['__init__'][1:] == list(inspect.signature(sb.HMR.__init__).parameters)[1:11]
-    tree = ast.parse(open('/root/reference/camcalib/model.py').read())
-    cls = [n for n in tree.body if isinstance(n, ast.ClassDef) and n.name == 'CameraRegressorNetwork'][0]
-    fns = {f.name: [a.arg for a in f.args.args] for f in cls.body if isinstance(f, ast.FunctionDef)}
-    assert fns['__init__'][1:] == list(inspect.signature(sb.CameraRegressorNetwork.__init__).parameters)[1:]
+    """Argument lists of the reference's drop-in classes, parsed from its sources into tests/golden/reference_tables.json
+    (tests/golden/reference_wrappers.py), equal the product's literally."""
+    import json
+    with open(os.path.join(ROOT, 'tests', 'golden', 'reference_tables.json')) as fh:
+        ref = json.load(fh)['signatures']
+    assert ref['HMR.forward'] == list(inspect.signature(sb.HMR.forward).parameters)[1:8]
+    assert ref['HMR.__init__'] == list(inspect.signature(sb.HMR.__init__).parameters)[1:11]
+    assert ref['CameraRegressorNetwork.__init__'] == list(inspect.signature(sb.CameraRegressorNetwork.__init__).parameters)[1:]
+    assert ref['CameraRegressorNetwork.forward'] == list(inspect.signature(sb.CameraRegressorNetwork.forward).parameters)[1:]
 
 
 @pytest.mark.parametrize('backbone', ['resnet50', 'resnet34', 'hrnet_w32-conv', 'hrnet_w32-interp'])

@@ -44,16 +44,12 @@ def test_joint_map_tables():
 
 
 def test_reference_name_tables_agree():
-    """If /root/reference is mounted (dev container), the restated tables equal the reference's own."""
-    path = '/root/reference/spec/constants.py'
-    if not os.path.exists(path):
-        pytest.skip('reference not mounted')
-    ns = {}
-    src = open(path).read()
-    exec(compile(src.split('# Permutation of SMPL pose parameters')[0].replace('import numpy as np', ''), path, 'exec'),
-         {'np': np}, ns)
-    assert ns['JOINT_NAMES'] == oc.JOINT_NAMES and ns['JOINT_MAP'] == oc.JOINT_MAP
-    assert ns['H36M_TO_J14'] == oc.H36M_TO_J14 and ns['IMG_NORM_MEAN'] == oc.IMG_NORM_MEAN
+    """The restated tables equal the reference's own (spec/constants.py), as recorded in tests/golden/reference_tables.json."""
+    import json
+    with open(os.path.join(GOLD, 'reference_tables.json')) as fh:
+        ref = json.load(fh)
+    assert ref['JOINT_NAMES'] == oc.JOINT_NAMES and ref['JOINT_MAP'] == oc.JOINT_MAP
+    assert ref['H36M_TO_J14'] == oc.H36M_TO_J14 and ref['IMG_NORM_MEAN'] == oc.IMG_NORM_MEAN
 
 
 def test_rot6d_orthonormal():

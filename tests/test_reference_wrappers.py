@@ -1,18 +1,18 @@
 """Pins the oracle's wrapper layer to OUTPUTS OF THE REFERENCE ITSELF (SURVEY.md 8c; VERDICT r1 item 3).
 
-tests/golden/reference_wrappers.py executes the unmodified /root/reference/camcalib/model.py, spec/models/hmr.py,
-camcalib/cam_utils.py and spec/utils/cam_params.py (with ``pare`` -- un-vendored, not installable -- stubbed in sys.modules
-by the oracle's restatements of its internals).  Here:
-
-* with /root/reference mounted (build container): the live reference wrappers and oracle/models.py + oracle/geometry.py are
-  run on the same seeded weights / inputs and must agree BIT FOR BIT, and the live run must reproduce the committed fixture;
-* everywhere (the GPU box has no /root/reference): the oracle must reproduce tests/golden/reference_wrappers.npz, the
-  committed output of that reference run, to fp32 round-off (a few ulps: the fixture may have been made on another CPU) --
-  the oracle's wrapper layer is checked against the reference's own code, not against itself.  The CUDA path is compared
-  with the same fixture in tests/test_gpu_parity.py::test_against_reference_wrapper_fixture.
+tests/golden/reference_wrappers.py executes the unmodified camcalib/model.py, spec/models/hmr.py, camcalib/cam_utils.py and
+spec/utils/cam_params.py of the original SPEC repository (with ``pare`` -- un-vendored, not installable -- stubbed in
+sys.modules by the oracle's restatements of its internals) and records what they produced: tests/golden/reference_wrappers.npz
+and, at a second set of seeds, tests/golden/reference_wrappers_alt_seeds.npz (vertices sampled), plus the reference's bin
+ranges in tests/golden/reference_tables.json.  Here the oracle must reproduce those recorded outputs to fp32 round-off (a few
+ulps: the fixtures may have been made on another CPU) -- the oracle's wrapper layer is checked against the reference's own code,
+not against itself.  The CUDA path is compared with the same fixture in
+tests/test_gpu_parity.py::test_against_reference_wrapper_fixture.
 
 What this does NOT pin: the internals behind the stubs (pare's backbones / HMRHead / SMPL, smplx's LBS), which remain
 restated from the published algorithms (oracle/__init__.py)."""
+import json
+
 import numpy as np
 import pytest
 import torch
@@ -26,21 +26,22 @@ def fixture():
 
 
 @pytest.fixture(scope='module')
-def live():
-    if not rw.reference_available():
-        pytest.skip('reference not mounted')
-    return rw.load_reference()
+def alt_fixture():
+    return np.load(rw.ALT_FIXTURE)
 
 
-def _same(name, got, want, exact=True):
-    """exact: same process, same thread count, same torch CPU kernels on both sides -> bit equality.  Against the COMMITTED
-    fixture (possibly made on another CPU / thread count, where the GEMM blocking and hence the fp32 summation order differ)
-    the bound is a few fp32 ulps: 2e-6 + 2e-6*|ref|, three orders below the north-star tolerances."""
+@pytest.fixture(scope='module')
+def tables():
+    with open(rw.TABLES) as fh:
+        return json.load(fh)
+
+
+def _same(name, got, want):
+    """Against a COMMITTED fixture (possibly made on another CPU / thread count, where the GEMM blocking and hence the fp32
+    summation order differ) the bound is a few fp32 ulps: 2e-6 + 2e-6*|ref|, three orders below the north-star tolerances."""
     assert got.shape == want.shape and got.dtype == want.dtype, (name, got.shape, want.shape, got.dtype, want.dtype)
     if got.dtype.kind in 'US':
         assert list(got) == list(want), name
-    elif exact:
-        assert np.array_equal(got, want), f'{name}: max abs diff {np.abs(got.astype(np.float64) - want.astype(np.float64)).max():.3e}'
     else:
         err = np.abs(got.astype(np.float64) - want.astype(np.float64))
         tol = 2e-6 + 2e-6 * np.abs(want.astype(np.float64))
@@ -53,24 +54,26 @@ def _same(name, got, want, exact=True):
 def test_oracle_reproduces_reference_fixture(fixture, case):
     """oracle == committed outputs of the reference's own wrapper code (to fp32 round-off, see _same)."""
     torch.set_num_threads(4)
-    seed = 40 + list(rw.CASES).index(case)
+    seed = rw.SEED0 + list(rw.CASES).index(case)
     got = rw.run_oracle_case(rw.CASES[case], seed)
     keys = [k[len(case) + 1:] for k in fixture.files if k.startswith(case + '/')]
     assert sorted(keys) == sorted(got), (sorted(keys), sorted(got))
     for k in keys:
-        _same(f'{case}/{k}', got[k], fixture[f'{case}/{k}'], exact=False)
+        _same(f'{case}/{k}', got[k], fixture[f'{case}/{k}'])
 
 
 @pytest.mark.parametrize('case', list(rw.CASES))
-def test_live_reference_wrappers_equal_oracle_and_fixture(live, fixture, case, tmp_path):
+def test_live_reference_wrappers_equal_oracle_and_fixture(alt_fixture, case):
+    """oracle == outputs recorded from a live run of the reference's wrapper code at a second set of seeds (weights and
+    inputs), vertices on a fixed sample (rw.ALT_VERTEX_IDS)."""
     torch.set_num_threads(4)
-    seed = 40 + list(rw.CASES).index(case)
-    ref_out = rw.run_reference_case(live, rw.CASES[case], seed, str(tmp_path))
-    ora_out = rw.run_oracle_case(rw.CASES[case], seed)
-    assert sorted(ref_out) == sorted(ora_out)
-    for k in ref_out:
-        _same(f'live {case}/{k}', ora_out[k], ref_out[k])
-        _same(f'fixture {case}/{k}', ref_out[k], fixture[f'{case}/{k}'], exact=False)
+    assert np.array_equal(alt_fixture['vertex_ids'], rw.ALT_VERTEX_IDS)
+    seed = rw.ALT_SEED0 + list(rw.CASES).index(case)
+    got = rw.alt_sample(rw.run_oracle_case(rw.CASES[case], seed))
+    keys = [k[len(case) + 1:] for k in alt_fixture.files if k.startswith(case + '/')]
+    assert sorted(keys) == sorted(got), (sorted(keys), sorted(got))
+    for k in keys:
+        _same(f'{case}/{k}', got[k], alt_fixture[f'{case}/{k}'])
 
 
 def test_reference_output_contract(fixture):
@@ -83,13 +86,12 @@ def test_reference_output_contract(fixture):
     assert (K[:, 2, 2] == 0).all() and (K[:, 0, 0] == K[:, 1, 1]).all()        # cam_params.py:39-46 leaves K[2,2] = 0
 
 
-def test_reference_bins_match_oracle_ranges(live):
+def test_reference_bins_match_oracle_ranges(tables):
     """The soft-argmax ranges the oracle hard-codes are the end points of the reference's own bin tables
-    (cam_utils.py:39,55,128-133)."""
+    (cam_utils.py:39,55,128-133), as recorded in tests/golden/reference_tables.json."""
     from oracle import geometry as og
-    cu = live['cam_utils']
-    assert float(np.min(cu.vfov_bins)) == og.VFOV_MIN and float(np.max(cu.vfov_bins)) == og.VFOV_MAX
-    assert float(np.min(cu.pitch_bins)) == og.PITCH_MIN and float(np.max(cu.pitch_bins)) == og.PITCH_MAX
+    assert tables['bins']['vfov_bins'] == [og.VFOV_MIN, og.VFOV_MAX]
+    assert tables['bins']['pitch_bins'] == [og.PITCH_MIN, og.PITCH_MAX]
 
 
 def test_product_decode_formula_matches_reference_fixture(fixture):
