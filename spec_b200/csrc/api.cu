@@ -211,8 +211,7 @@ extern "C" int specb200_trunk_create(specb200_trunk_t** out, const specb200_op_t
         if (o.type == SPECB200_OP_CONV) {
             if (o.wslot < 0 || o.wslot >= n_wslots) { set_error("trunk_create: bad wslot"); delete t; return 1; }
             t->wslot_cin[o.wslot] = o.cin;
-            const char* np = getenv("SPECB200_NO_PAIR");
-            const bool pair_ok = o.pair && t->prec != PREC_F32 && !(np && np[0] == '1') && o.cin == 32 && o.cout == 32 && o.kh == 3 &&
+            const bool pair_ok = o.pair && t->prec != PREC_F32 && o.cin == 32 && o.cout == 32 && o.kh == 3 &&
                                  o.kw == 3 && o.stride == 1 && o.pad == 1 && o.dst_coff == 0 && t->buf_ch[o.src] == 32 &&
                                  t->buf_ch[o.dst] == 32 && (o.src2 < 0 || t->buf_ch[o.src2] == 32);
             t->wslot_pair[o.wslot] = pair_ok ? 1 : 0;
@@ -223,8 +222,7 @@ extern "C" int specb200_trunk_create(specb200_trunk_t** out, const specb200_op_t
         bool ok = t->prec != PREC_F32 && o.type == SPECB200_OP_CONV && o.src == 0 && o.kh == 7 && o.kw == 7 && o.stride == 2 &&
                   o.pad == 3 && o.cout == 64 && o.relu && o.src2 < 0 && o.dst_coff == 0 && t->buf_ch[o.dst] == 64;
         for (size_t i = 1; i < t->ops.size() && ok; ++i) ok = t->ops[i].src != 0 && t->ops[i].src2 != 0;
-        const char* e = getenv("SPECB200_NO_STEM7");
-        if (ok && !(e && e[0] == '1')) t->stem7_slot = o.wslot;
+        if (ok) t->stem7_slot = o.wslot;
     }
     trunk_find_bottlenecks(t);
     *out = t;
@@ -430,12 +428,6 @@ static int trunk_forward_impl(specb200_trunk_t* t, const float* images, int32_t 
                     p.out_ld = t->buf_ch[o.dst]; p.out_coff = o.dst_coff;
                     p.res_ld = o.src2 >= 0 ? t->buf_ch[o.src2] : 0;
                     p.relu = o.relu;
-                    // second TMA producer thread for the weight tiles: one thread that waits, arms and issues two loads per k-block
-                    // tops out at ~350 ns per block (tools/tma_mcast_test.cu); splitting A and B over two threads gave -7..-11 % on
-                    // the 3x3 CTA-pair convs and passed the parity suite on B200 (round 2).  SPECB200_SPLIT_PRODUCER=0: A/B baseline
-                    static int split_prod = -1;
-                    if (split_prod < 0) { const char* e = getenv("SPECB200_SPLIT_PRODUCER"); split_prod = (e && e[0] == '0') ? 0 : 1; }
-                    p.split_producer = split_prod;
                     if (pair) { p.W /= 2; p.Wo /= 2; p.M /= 2; p.Cin = 64; p.Cout = 64; p.out_ld = 64; p.res_ld = o.src2 >= 0 ? 64 : 0; }
                     const bool ok = (t->prec == PREC_F32) ? conv_f32_launch(p, cw, s)
                                     : (conv_halo_applicable(p, cw) ? conv_halo_launch(p, cw, t->prec, s) : conv_tc_launch(p, cw, t->prec, s));

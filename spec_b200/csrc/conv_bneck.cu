@@ -493,9 +493,6 @@ bool bneck_launch_t(const BottleneckArgs& a, cudaStream_t s) {
 }  // namespace
 
 bool bottleneck_applicable(const BottleneckArgs& a) {
-    static int off = -1;
-    if (off < 0) { const char* e = getenv("SPECB200_NO_BNECK"); off = (e && e[0] == '1') ? 1 : 0; }
-    if (off) return false;
     const bool ds = a.wd != nullptr;
     const int cin = ds ? 64 : 256;
     auto ok16 = [](const ConvWeights* w, int cout, int cin_, int k) {

@@ -468,11 +468,9 @@ bool conv_stem7_launch(const float* img, void* out, const ConvWeights& w, int N,
     const int tiles_h = (Ho + ST_TH - 1) / ST_TH, tiles_w = (Wo + ST_TW - 1) / ST_TW;
     const long long total = static_cast<long long>(N) * tiles_h * tiles_w;
     if (total > 0x7fffffffLL) { set_error("conv_stem7: too many tiles"); return false; }
-    static int v1 = -1;                                          // SPECB200_STEM_V1=1: the first (non-pipelined) kernel, for A/B runs
-    if (v1 < 0) { const char* e = getenv("SPECB200_STEM_V1"); v1 = (e && e[0] == '1') ? 1 : 0; }
     // the TMA-fed kernel needs 16-byte aligned image rows (W % 4 == 0) and an image at least one box (40 x 21) large;
     // other shapes keep the first kernel
-    if (!v1 && (W % 4) == 0 && W >= STP_RP && H >= ST_PR && (reinterpret_cast<uintptr_t>(img) & 15) == 0) {
+    if ((W % 4) == 0 && W >= STP_RP && H >= ST_PR && (reinterpret_cast<uintptr_t>(img) & 15) == 0) {
         CUtensorMap tmap_out, tmap_img;
         if (!make_tmap_nhwc(&tmap_out, out, 64, Wo, Ho, N, ST_TW, ST_TH)) return false;
         if (!make_tmap_image_f32(&tmap_img, img, W, H, N)) return false;

@@ -24,10 +24,15 @@
 //              -> ReLU -> 16-bit.  EPI_TMA: the residual tile is TMA-loaded into the (by then free)
 //              pipeline smem, combined in place, and the finished tile leaves through a TMA store --
 //              fully coalesced 128-byte lines in both directions.  BLOCK_N = 32 keeps direct stores.
-//   warp 4     TMA producer (A and B); owns the TMEM allocation.
+//   warp 4     TMA producer (A, and B in the gather modes); owns the TMEM allocation.
 //   warp 5     MMA issuer: one thread issues tcgen05.mma (M=128, N=BLOCK_N, K=16) x4 per stage and
 //              commits stage release / accumulator-ready to mbarriers.
 //   warps 6-9  second epilogue group: in the TMA-store epilogue they convert the upper half of the columns.
+//              In the TMA-fed modes warp 6 first issues the weight tiles (second producer).
+//
+// Second producer: one thread that waits, arms and issues two TMA loads per k-block tops out at ~350 ns per block
+// (tools/tma_mcast_test.cu); issuing A and B from two threads gave -7..-11 % on the 3x3 CTA-pair convs (B200, round 2).
+// All three tcgen05 conv kernels split their producers this way.
 //
 // BLOCK_N = 256 (3x3 convs with Cout >= 256): at 128 x 128 tiles the tensor pipe consumes 128 B/cycle of operands,
 // so covering ~1.5k cycles of TMA latency needs ~190 KB in flight -- more than one SM's smem; a 128 x 256 tile needs
@@ -138,10 +143,10 @@ conv_tc_kernel(const ConvParams p, const __grid_constant__ ConvTcMaps maps, int 
         const int t = q4 * 32 + lane;                            // tile row == TMEM lane
         const long long r = static_cast<long long>(m_tile) * TILE_M + t;
         const bool row_ok = r < p.M;
-        // ---------------- optional second TMA producer (experiment, ConvParams::split_producer): warp 6 issues the weight tiles
-        // while warp 4 issues A; its epilogue share starts afterwards (every load is issued long before the last MMA retires)
+        // ---------------- second TMA producer: warp 6 issues the weight tiles while warp 4 issues A; its epilogue share starts
+        // afterwards (every load is issued long before the last MMA retires)
         if constexpr (A_MODE == A_TILED || A_MODE == A_IM2COL) {
-            if (p.split_producer && warp == 6) {
+            if (warp == 6) {
                 if (lane == 0) {
                     for (int kb = 0; kb < num_kb; ++kb) {
                         const int s = kb % STAGES;
@@ -351,7 +356,7 @@ conv_tc_kernel(const ConvParams p, const __grid_constant__ ConvTcMaps maps, int 
                 const int it = kb / STAGES;
                 mbar_wait(bar_empty + s * 8, (it & 1) ^ 1);
                 mbar_arrive_expect_tx(bar_full + s * 8, tx_bytes);
-                if (!(p.split_producer && (A_MODE == A_TILED || A_MODE == A_IM2COL)))
+                if constexpr (A_MODE == A_GATHER || A_MODE == A_STEM)
                     tma_load_2d(b_base + s * L::B_STAGE_BYTES, &maps.b, bar_full + s * 8, kb * TILE_K, n0);
                 if constexpr (A_MODE == A_TILED) {
                     tma_load_2d(a_base + s * A_STAGE_BYTES, &maps.a, bar_full + s * 8, kb * TILE_K, m_tile * TILE_M);
@@ -490,14 +495,13 @@ conv_tcp_kernel(const ConvParams p, const __grid_constant__ ConvTcMaps maps, int
     const uint32_t tmem_base = *tmem_ptr_s;
 
     if (warp == 0) {
-        // ================= TMA producer
+        // ================= TMA producer (A; arms the full barrier for both operands)
         if (lane == 0) {
             constexpr uint32_t tx_bytes = L::B_STAGE_BYTES + A_STAGE_BYTES;
             const int hw = p.Ho * p.Wo;
             uint32_t kc = 0;
             for (int tile = blockIdx.x; tile < total_tiles; tile += gridDim.x) {
-                const int n_tile = tile % n_tiles, m_tile = tile / n_tiles;
-                const int n0 = n_tile * BLOCK_N;
+                const int m_tile = tile / n_tiles;
                 int pw = 0, ph = 0, pn = 0;
                 if constexpr (A_MODE == A_IM2COL) {
                     const long long r0 = static_cast<long long>(m_tile) * TILE_M;
@@ -511,7 +515,6 @@ conv_tcp_kernel(const ConvParams p, const __grid_constant__ ConvTcMaps maps, int
                     const uint32_t s = kc % STAGES, it = kc / STAGES;
                     mbar_wait(bar_empty + s * 8, (it & 1) ^ 1);
                     mbar_arrive_expect_tx(bar_full + s * 8, tx_bytes);
-                    if (!p.split_producer) tma_load_2d(b_base + s * L::B_STAGE_BYTES, &maps.b, bar_full + s * 8, kb * TILE_K, n0);
                     if constexpr (A_MODE == A_TILED) {
                         tma_load_2d(a_base + s * A_STAGE_BYTES, &maps.a, bar_full + s * 8, kb * TILE_K, m_tile * TILE_M);
                     } else {
@@ -526,8 +529,8 @@ conv_tcp_kernel(const ConvParams p, const __grid_constant__ ConvTcMaps maps, int
             }
         }
         __syncwarp();
-    } else if (warp == 3 && p.split_producer) {
-        // ================= second producer (experiment): the weight tiles, same stage / phase sequence as warp 0
+    } else if (warp == 3) {
+        // ================= second producer: the weight tiles, same stage / phase sequence as warp 0
         if (lane == 0) {
             uint32_t kc = 0;
             for (int tile = blockIdx.x; tile < total_tiles; tile += gridDim.x) {
@@ -746,10 +749,7 @@ int conv_tc_pick_block_n(int cout, int K) {
     if (cout <= 64) return 64;
     // 128 x 256 tiles when there are >= 4 k-blocks to amortise the wider epilogue (measured: K = 64 / 128 expansions
     // are faster at N = 128, everything with K >= 256 and Cout % 256 == 0 is faster at N = 256)
-    if (cout >= 256 && (cout % 256) == 0 && K >= 256) {
-        const char* e = getenv("SPECB200_NO_N256");
-        if (!(e && e[0] == '1')) return 256;
-    }
+    if (cout >= 256 && (cout % 256) == 0 && K >= 256) return 256;
     return 128;
 }
 
@@ -761,11 +761,7 @@ bool conv_tc_make_weight_tmap(ConvWeights& w) {
     return true;
 }
 
-static int g_force_gather = -1;     // SPECB200_FORCE_GATHER=1 disables the TMA im2col path (debug / A-B test)
-static int g_no_persist = -1;       // SPECB200_NO_PERSIST=1 keeps the one-tile-per-CTA kernel (A-B test)
 static int g_num_sms = 0;
-
-static int g_use_2cta = -1;         // SPECB200_NO_2CTA=1 keeps the one-CTA persistent kernel
 
 // CTA-pair (cta_group::2) persistent kernel: 256 x BLOCK_N tiles over clusters of two CTAs
 template <typename T, int BLOCK_N, int STAGES>
@@ -820,11 +816,10 @@ static bool launch_persistent(const ConvParams& p, const ConvTcMaps& maps, int m
 template <typename T, int BLOCK_N, int STAGES>
 static bool launch_cfg(const ConvParams& p, const ConvWeights& w, cudaStream_t s) {
     using L = ConvTcSmem<BLOCK_N, STAGES>;
-    if (g_force_gather < 0) { const char* e = getenv("SPECB200_FORCE_GATHER"); g_force_gather = (e && e[0] == '1') ? 1 : 0; }
     int mode = A_GATHER;
     if (w.kwp > 0) mode = A_STEM;
     else if (p.kh == 1 && p.kw == 1 && p.stride == 1 && p.pad == 0 && (p.Cin % TILE_K) == 0) mode = A_TILED;
-    else if ((p.Cin % TILE_K) == 0 && !g_force_gather) mode = A_IM2COL;
+    else if ((p.Cin % TILE_K) == 0) mode = A_IM2COL;
     const int m_tiles = (p.M + TILE_M - 1) / TILE_M;
     const int n_tiles = (p.Cout + BLOCK_N - 1) / BLOCK_N;
     ConvTcMaps maps;
@@ -840,23 +835,13 @@ static bool launch_cfg(const ConvParams& p, const ConvWeights& w, cudaStream_t s
         if (p.res != nullptr &&
             !make_tmap_2d(&maps.res, p.res, static_cast<uint64_t>(p.M), static_cast<uint64_t>(p.res_ld), static_cast<uint64_t>(p.res_ld), TILE_M)) return false;
     }
-    if (g_no_persist < 0) { const char* e = getenv("SPECB200_NO_PERSIST"); g_no_persist = (e && e[0] == '1') ? 1 : 0; }
     if constexpr (BLOCK_N == 64 || BLOCK_N == 128 || BLOCK_N == 256) {
         // k>1 convs at N<=128: two co-resident one-tile CTAs feed the tensor pipe better than one persistent CTA (measured);
-        // at N=256 the operand bytes per MMA cycle drop to 96 B and the persistent kernel (overlapped epilogue) wins.
-        if (g_use_2cta < 0) { const char* e = getenv("SPECB200_NO_2CTA"); g_use_2cta = (e && e[0] == '1') ? 0 : 1; }
-        static int pair128 = -1;           // SPECB200_PAIR128=1: CTA pairs also for 128-wide tiles with K >= 256 (experiment)
-        if (pair128 < 0) { const char* e = getenv("SPECB200_PAIR128"); pair128 = (e && e[0] == '1') ? 1 : 0; }
+        // at N=256 the operand bytes per MMA cycle drop to 96 B and the persistent kernels (overlapped epilogue) win.
         const bool tma_fed = (mode == A_TILED || mode == A_IM2COL) && (p.Cout & 63) == 0 && p.Cout <= 2048;
-        if constexpr (BLOCK_N == 128) {
-            if (!g_no_persist && tma_fed && g_use_2cta && pair128 && m_tiles >= 2 && p.K >= 256)
-                return launch_pair<T, 128, 6>(p, maps, w, mode, m_tiles, n_tiles, s);
-        }
         const bool one_tile_better = p.kh * p.kw > 1 && BLOCK_N < 256;
-        if (!g_no_persist && !one_tile_better && tma_fed) {
-            if constexpr (BLOCK_N == 256) {
-                if (g_use_2cta && m_tiles >= 2) return launch_pair<T, 256, 4>(p, maps, w, mode, m_tiles, n_tiles, s);
-            }
+        if (tma_fed && !one_tile_better) {
+            if (BLOCK_N == 256 && m_tiles >= 2) return launch_pair<T, 256, 4>(p, maps, w, mode, m_tiles, n_tiles, s);
             return launch_persistent<T, BLOCK_N, (BLOCK_N == 256 ? 3 : (BLOCK_N == 128 ? 4 : 6))>(p, maps, mode, m_tiles, n_tiles, s);
         }
     }

@@ -84,14 +84,13 @@ conv_tcp2_kernel(const ConvParams p, const __grid_constant__ ConvTcMaps maps, in
     const uint32_t tmem_base = *tmem_ptr_s;
 
     if (warp == 0) {
-        // ================= TMA producer (one per CTA; completion counted on the leader's full barrier)
+        // ================= TMA producer (A; one per CTA, arms the leader's full barrier for both operands)
         if (lane == 0) {
             constexpr uint32_t tx_bytes = L::B_STAGE_BYTES + A_STAGE_BYTES;
             const int hw = p.Ho * p.Wo;
             uint32_t kc = 0;
             for (int tile = first_tile; tile < total_tiles; tile += tile_step) {
-                const int n_tile = tile % n_tiles, m_tile = (tile / n_tiles) * 2 + static_cast<int>(rank);
-                const int nrow0 = n_tile * BLOCK_N + static_cast<int>(rank) * (BLOCK_N / 2);
+                const int m_tile = (tile / n_tiles) * 2 + static_cast<int>(rank);
                 int pw = 0, ph = 0, pn = 0;
                 if constexpr (A_MODE == A_IM2COL) {
                     const long long r0 = static_cast<long long>(m_tile) * TILE_M;
@@ -106,7 +105,6 @@ conv_tcp2_kernel(const ConvParams p, const __grid_constant__ ConvTcMaps maps, in
                     mbar_wait(bar_empty + s * 8, (it & 1) ^ 1);                  // own stage released (multicast commit)
                     const uint32_t lead_full = mapa_u32(bar_full + s * 8, 0);
                     mbar_arrive_expect_tx_cluster(lead_full, tx_bytes);
-                    if (!p.split_producer) tma_load_2d_2sm(b_base + s * L::B_STAGE_BYTES, &maps.b, lead_full, kb * TILE_K, nrow0);
                     if constexpr (A_MODE == A_TILED) {
                         tma_load_2d_2sm(a_base + s * A_STAGE_BYTES, &maps.a, lead_full, kb * TILE_K, m_tile * TILE_M);
                     } else {
@@ -121,8 +119,8 @@ conv_tcp2_kernel(const ConvParams p, const __grid_constant__ ConvTcMaps maps, in
             }
         }
         __syncwarp();
-    } else if (warp == 3 && p.split_producer) {
-        // ================= second producer (experiment): the weight half-tiles, same stage / phase sequence as warp 0.
+    } else if (warp == 3) {
+        // ================= second producer: the weight half-tiles, same stage / phase sequence as warp 0.
         // Bytes that land before warp 0 has armed the barrier only make the tx-count transiently negative.
         if (lane == 0) {
             uint32_t kc = 0;

@@ -191,9 +191,7 @@ maxpool_tma_kernel(const __grid_constant__ CUtensorMap tmap_in, const __grid_con
 }
 
 bool maxpool3x3s2_launch(const void* in, void* out, int N, int H, int W, int C, int Ho, int Wo, int prec, cudaStream_t s, bool nonneg_input) {
-    static int no_tma = -1;                                              // SPECB200_NO_POOL_TMA=1: the L1 re-read kernel (A/B baseline)
-    if (no_tma < 0) { const char* e = getenv("SPECB200_NO_POOL_TMA"); no_tma = (e && e[0] == '1') ? 1 : 0; }
-    if (!no_tma && nonneg_input && C == 64 && prec != PREC_F32 && H >= MP_PH && W >= MP_PW) {
+    if (nonneg_input && C == 64 && prec != PREC_F32 && H >= MP_PH && W >= MP_PW) {
         CUtensorMap tin, tout;
         if (!make_tmap_nhwc(&tin, in, 64, W, H, N, MP_PW, MP_PH)) return false;
         if (!make_tmap_nhwc(&tout, out, 64, Wo, Ho, N, MP_TW, MP_TH)) return false;

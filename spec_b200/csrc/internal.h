@@ -24,7 +24,6 @@ struct ConvParams {
     int M;               // N*Ho*Wo
     int out_ld, out_coff, res_ld;
     int relu;
-    int split_producer;  // experiment (SPECB200_SPLIT_PRODUCER=1): the weight-tile TMA loads are issued by a second producer thread
 };
 
 // Packed weights of one conv, owned by the trunk handle.

@@ -371,15 +371,7 @@ class HMR(nn.Module):
         graph.replay()
         return {k: v.clone() for k, v in outs.items()}             # fresh tensors owned by the caller
 
-    def run_trunk(self, images):
-        """Enqueue only the backbone (pooled features land in the head's input rows); pair with ``_forward_impl(...,
-        _skip_trunk=True)``.  Lets a caller overlap this trunk with other work (SPECPipeline runs CamCalib beside it)."""
-        _lib.require_device(images)
-        self._ensure(images.device)
-        ws = self._workspace(images.shape[0], images.device)
-        self.backbone.run(images, pooled=ws.data_ptr(), pooled_ld=self._x_ld)
-
-    def _forward_impl(self, images, cam_rotmat, cam_intrinsics, bbox_scale, bbox_center, img_w, img_h, _out, _skip_trunk=False):
+    def _forward_impl(self, images, cam_rotmat, cam_intrinsics, bbox_scale, bbox_center, img_w, img_h, _out):
         _lib.require_device(images)
         dev = images.device
         B = images.shape[0]
@@ -399,8 +391,7 @@ class HMR(nn.Module):
         ih = self._f32(img_h, B, dev, ())
         ws = self._workspace(B, dev)
         # trunk writes the pooled feature straight into the head's input rows
-        if not _skip_trunk:
-            self.backbone.run(images, pooled=ws.data_ptr(), pooled_ld=self._x_ld)
+        self.backbone.run(images, pooled=ws.data_ptr(), pooled_ld=self._x_ld)
         o = _lib.HmrOutputs()
         result = {}
         for key in _lib.OUTPUT_KEYS:

@@ -27,18 +27,11 @@ def unpack_record(record):
 
 
 class SPECPipeline:
-    def __init__(self, camcalib: CameraRegressorNetwork, hmr: HMR, use_graph=True, overlap_trunks=None):
+    def __init__(self, camcalib: CameraRegressorNetwork, hmr: HMR, use_graph=True):
         if not (hmr.use_cam and hmr.use_cam_feats):
             raise ValueError('the SPEC pipeline uses HMR(use_cam=True, use_cam_feats=True) (spec/tester.py:53-59)')
         self.camcalib, self.hmr = camcalib, hmr
         self.use_graph = use_graph
-        # The two trunks are independent until the head needs (R, K); running CamCalib on a side stream beside the HMR trunk
-        # (fork/join captured in the graph) was MEASURED SLOWER on B200 (12.5 vs 8.2 ms/step at B=256): the conv kernels are
-        # persistent one-CTA-per-SM kernels with ~200 KB of smem, so two of them time-slice instead of back-filling.  Off by
-        # default; SPECB200_OVERLAP_TRUNKS=1 or overlap_trunks=True enables it for experiments.
-        import os
-        self.overlap_trunks = (os.environ.get('SPECB200_OVERLAP_TRUNKS', '0') == '1') if overlap_trunks is None else overlap_trunks
-        self._side = None
         self._graph = None
         self._static = None
         self._keep = None
@@ -51,22 +44,12 @@ class SPECPipeline:
         out = {k: (record[:, _OFFSETS[k][0]:_OFFSETS[k][0] + _OFFSETS[k][1]].view((B,) + _OFFSETS[k][2]), RECORD_FLOATS)
                for k in _lib.OUTPUT_KEYS}
         o, n, _ = _OFFSETS['cam_angles']
-        if not self.overlap_trunks:
-            angles, R, K, _ = self.camcalib.predict_camera(images, img_h, img_w)
-            record[:, o:o + n].copy_(angles)
-            self.hmr(images, R, K, bbox_scale, bbox_center, img_w, img_h, _out=out)
-            return record
-        main = torch.cuda.current_stream(images.device)
-        if self._side is None or self._side.device != images.device:
-            self._side = torch.cuda.Stream(device=images.device)
-        side = self._side
-        side.wait_stream(main)
-        with torch.cuda.stream(side):
-            angles, R, K, _ = self.camcalib.predict_camera(images, img_h, img_w)
-            record[:, o:o + n].copy_(angles)
-        self.hmr.run_trunk(images)
-        main.wait_stream(side)
-        self.hmr._forward_impl(images, R, K, bbox_scale, bbox_center, img_w, img_h, out, _skip_trunk=True)
+        # The two trunks run one after the other on one stream.  CamCalib on a side stream beside the HMR trunk was measured
+        # slower on B200 (12.5 vs 8.2 ms/step at B=256): the conv kernels are persistent one-CTA-per-SM kernels with ~200 KB
+        # of smem, so two of them time-slice instead of back-filling.
+        angles, R, K, _ = self.camcalib.predict_camera(images, img_h, img_w)
+        record[:, o:o + n].copy_(angles)
+        self.hmr(images, R, K, bbox_scale, bbox_center, img_w, img_h, _out=out)
         return record
 
     @torch.no_grad()

@@ -68,17 +68,17 @@ def _mini_ref(t, x, dtype, res):
 
 CONV_CASES = [
     # cmid, cout, k, stride, pad, res, H, W, B      what it exercises
-    (64, 64, 1, 1, 0, False, 16, 16, 2),            # 1x1: TMA A path, 1 k-block, BLOCK_N=64
-    (256, 128, 1, 1, 0, True, 12, 20, 3),           # 1x1 TMA A, 4 k-blocks, BLOCK_N=128, residual, ragged M
-    (64, 64, 3, 1, 1, False, 14, 14, 2),            # 3x3 gather, padding, 9 k-blocks
-    (128, 128, 3, 2, 1, False, 15, 17, 2),          # 3x3 stride 2, odd sizes
-    (64, 256, 1, 2, 0, False, 14, 14, 2),           # strided 1x1 (downsample) -> gather path
-    (32, 32, 3, 1, 1, True, 10, 10, 2),             # Cin=32 (HRNet): two taps per k-block, BLOCK_N=32
-    (64, 512, 1, 1, 0, False, 7, 7, 5),             # 4 N tiles
-    (64, 64, 3, 1, 1, True, 9, 23, 3),              # halo kernel, resident weights, ragged 8x14 tiles, residual
-    (128, 128, 3, 1, 1, True, 20, 30, 2),           # halo kernel, streamed weights (2 channel blocks), residual
-    (256, 256, 3, 1, 1, False, 16, 17, 1),          # halo kernel, N=256 (two epilogue sub-tiles), 4 channel blocks
-    (256, 512, 1, 1, 0, True, 9, 9, 3),             # persistent 1x1, N=256 tiles, residual
+    (64, 64, 1, 1, 0, False, 16, 16, 2),            # 1x1: tiled TMA A, 1 k-block, BLOCK_N=64, persistent kernel
+    (256, 128, 1, 1, 0, True, 12, 20, 3),           # 1x1 tiled TMA A, 4 k-blocks, BLOCK_N=128, persistent kernel, residual, ragged M
+    (64, 64, 3, 1, 1, False, 14, 14, 2),            # halo kernel, 8x14 tiles, padding
+    (128, 128, 3, 2, 1, False, 15, 17, 2),          # 3x3 stride 2, odd sizes: TMA im2col A, one-tile kernel
+    (64, 256, 1, 2, 0, False, 14, 14, 2),           # strided 1x1 (downsample): TMA im2col A, persistent kernel, BLOCK_N=128 (K=64)
+    (32, 32, 3, 1, 1, True, 10, 10, 2),             # Cin=32 (HRNet), even width: pixel-pair view as a 64->64 conv, too narrow for the halo kernel -> im2col one-tile kernel
+    (64, 512, 1, 1, 0, False, 7, 7, 5),             # persistent kernel, 4 N tiles
+    (64, 64, 3, 1, 1, True, 9, 23, 3),              # halo kernel, ragged 4x30 tiles, residual
+    (128, 128, 3, 1, 1, True, 20, 30, 2),           # 3x3 TMA im2col A, one-tile kernel, BLOCK_N=128, residual
+    (256, 256, 3, 1, 1, False, 16, 17, 1),          # CTA-pair kernel, im2col A, N=256, 3 m-tiles: the second pair tile is half outside M
+    (256, 512, 1, 1, 0, True, 9, 9, 3),             # CTA-pair kernel, tiled A, N=256 tiles, residual, ragged M
     (32, 32, 3, 1, 1, True, 9, 11, 2),              # Cin=32 on an ODD width: the pixel-pair view does not apply -> gather-kernel fallback
     (512, 512, 3, 1, 1, False, 14, 14, 56),         # CTA-pair kernel, im2col A, K=4608: 43 pair-tiles x 2 n-tiles = 86 tiles on 74 clusters (multi-tile loop)
     (1024, 2048, 1, 1, 0, True, 7, 7, 200),         # CTA-pair kernel, 1x1: 39 pair-tiles x 8 n-tiles = 312 tiles on 74 clusters: the multi-tile loop + TMEM phase flips
