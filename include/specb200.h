@@ -56,6 +56,7 @@ typedef struct specb200_op {
 typedef struct specb200_trunk specb200_trunk_t;
 typedef struct specb200_camtail specb200_camtail_t;
 typedef struct specb200_hmrtail specb200_hmrtail_t;
+typedef struct specb200_body specb200_body_t;
 
 const char* specb200_last_error(void);
 int specb200_abi_version(void);
@@ -173,6 +174,28 @@ int specb200_hmrtail_forward(specb200_hmrtail_t* t, int32_t batch, void* workspa
 int64_t specb200_hmrtail_last_launches(specb200_hmrtail_t* t);
 void specb200_hmrtail_destroy(specb200_hmrtail_t* t);
 
+/* ---- SMPL body model: smplx.SMPL forward from caller-given parameters, as the evaluation side calls it
+ *      (/root/reference/spec/utils/compute_error.py:148-181: axis-angle pose, pose2rot=True; spec/trainer.py:249-254:
+ *      rotation matrices, pose2rot=False).  Same kernels as the HMR tail's SMPL stage.  Any number of body handles (e.g.
+ *      neutral, male, female) and HMR tail handles may live side by side. --------------------------------------------- */
+/* host, smplx layout: v_template [6890][3], shapedirs [6890][3][10], posedirs [207][20670], J_regressor [24][6890],
+ * lbs_weights [6890][24], parents [24] (the standard SMPL tree) */
+int specb200_body_create(specb200_body_t** out, const float* v_template, const float* shapedirs, const float* posedirs,
+                         const float* J_regressor, const float* lbs_weights, const int32_t* parents);
+int64_t specb200_body_workspace_bytes(specb200_body_t* t, int32_t batch);
+#define SPECB200_POSE_AXIS_ANGLE 0 /* pose_dev: [batch][72] axis-angle (global_orient first), smplx batch_rodrigues */
+#define SPECB200_POSE_ROTMAT 1     /* pose_dev: [batch][24][9] rotation matrices                                   */
+/* betas_dev [batch][10].  Outputs (device fp32, per-image strides in floats): verts [6890][3]; joints24 [24][3] = the posed
+ * kinematic joints (smplx's joints[:, :24]).  workspace_dev: 256-byte aligned, >= specb200_body_workspace_bytes. */
+int specb200_body_forward(specb200_body_t* t, int32_t batch, const float* betas_dev, const float* pose_dev, int32_t pose_kind,
+                          void* workspace_dev, int64_t workspace_bytes, float* verts_dev, int64_t ld_verts, float* joints24_dev,
+                          int64_t ld_joints24, void* stream);
+/* joints24_out_dev [batch][24][3] = rot . (J_regressor . verts) (compute_error.py:184-187: einsum('bik,ji->bjk')); verts_dev
+ * [batch][6890][3] with per-image stride ld_verts floats; rot_dev [batch][9] or NULL (no rotation). */
+int specb200_body_regress_joints(specb200_body_t* t, int32_t batch, const float* verts_dev, int64_t ld_verts, const float* rot_dev,
+                                 float* joints24_out_dev, void* stream);
+void specb200_body_destroy(specb200_body_t* t);
+
 /* ---- eval-side metrics on the device (SURVEY.md section 8f-1): replaces the J_regressor_h36m matmul, pelvis centring, MPJPE,
  *      numpy Procrustes (PA-MPJPE) and per-vertex error of /root/reference/spec/trainer.py:272-316 and
  *      /root/reference/spec/utils/compute_error.py:33-86 -------------------------------------------------------------- */
@@ -188,6 +211,24 @@ int specb200_eval_forward(specb200_eval_t* t, int32_t batch, const float* pred_v
                           const float* gt_keypoints14_dev, const float* gt_verts_dev, int64_t ld_gt, int32_t center_v2v,
                           void* workspace_dev, int64_t workspace_bytes, float* mpjpe_dev, float* pampjpe_dev, float* v2v_dev,
                           float* pred_keypoints14_dev, void* stream);
+/* joint_mapper_host: n_map (14 or 17) indices into the 17 joints: H36M_TO_J14, or H36M_TO_J17 (trainer.py:259-260). */
+int specb200_eval_create_mapped(specb200_eval_t** out, const float* J_regressor_h36m_host, const int32_t* joint_mapper_host,
+                                int32_t n_map);
+/* specb200_eval_forward plus: pred_rot_dev / gt_rot_dev ([batch][9] or NULL) rotate each mesh before the regression, centring
+ * and v2v (compute_error.py:164,186: the camera-frame metrics); gt_rot_dev also rotates given keypoints; per-joint
+ * distances before / after the Procrustes alignment, mpjpe_pj_dev / pampjpe_pj_dev [batch][n_map] (NULL to skip);
+ * gt keypoints and pred_keypoints are [batch][n_map][3]; n_map must equal the handle's mapper length. */
+int specb200_eval_forward_ex(specb200_eval_t* t, int32_t batch, const float* pred_verts_dev, int64_t ld_pred, const float* pred_rot_dev,
+                             const float* gt_keypoints_dev, const float* gt_verts_dev, int64_t ld_gt, const float* gt_rot_dev,
+                             int32_t center_v2v, void* workspace_dev, int64_t workspace_bytes, float* mpjpe_dev, float* pampjpe_dev,
+                             float* v2v_dev, float* pred_keypoints_dev, float* mpjpe_pj_dev, float* pampjpe_pj_dev, int32_t n_map,
+                             void* stream);
+/* Stateless: MPJPE / PA-MPJPE of already-regressed joints pred_dev, gt_dev [batch][n][3] (n = 14, 17 or 24), e.g. the 24 SMPL
+ * joints of specb200_body_*.  rot_pred_dev / rot_gt_dev ([batch][9] or NULL) rotate each side first; center != 0 subtracts
+ * joint 0 on both sides (compute_error.py:33-49 eval_j_24).  Per-joint outputs [batch][n] may be NULL. */
+int specb200_eval_joint_errors(int32_t batch, int32_t n, const float* pred_dev, const float* gt_dev, const float* rot_pred_dev,
+                               const float* rot_gt_dev, int32_t center, float* mpjpe_dev, float* pampjpe_dev, float* mpjpe_pj_dev,
+                               float* pampjpe_pj_dev, void* stream);
 void specb200_eval_destroy(specb200_eval_t* t);
 
 /* ---- input side on the device (SURVEY.md section 8f-2): uint8 frame -> network inputs, BIT-EXACT with the

@@ -13,11 +13,12 @@ from .backbone import get_backbone_info, resnet18, resnet34, resnet50, resnet101
 from .cam_utils import convert_preds_to_angles, decode_logits
 from .pipeline import (SPECPipeline, unpack_record, all_gather_records, shard_range, RecordGatherer, PeerGatherer, make_gatherer,
                        bind_process_to_gpu_numa, unbind_process)
-from .metrics import EvalMetrics
+from .metrics import EvalMetrics, SPECErrorEval, joint_errors
+from .body_model import BodyModel
 from .preprocess import Preprocessor, get_single_image_crop_demo, camcalib_transform
 
 __all__ = ['CameraRegressorNetwork', 'HMR', 'HMRHead', 'SMPLCamHead', 'SMPLHead', 'get_backbone_info',
            'resnet18', 'resnet34', 'resnet50', 'resnet101', 'hrnet_w32', 'hrnet_w48',
            'convert_preds_to_angles', 'decode_logits', 'SPECPipeline', 'unpack_record', 'all_gather_records',
-           'shard_range', 'RecordGatherer', 'PeerGatherer', 'make_gatherer', 'bind_process_to_gpu_numa', 'unbind_process', 'EvalMetrics', 'Preprocessor', 'get_single_image_crop_demo',
+           'shard_range', 'RecordGatherer', 'PeerGatherer', 'make_gatherer', 'bind_process_to_gpu_numa', 'unbind_process', 'EvalMetrics', 'SPECErrorEval', 'joint_errors', 'BodyModel', 'Preprocessor', 'get_single_image_crop_demo',
            'camcalib_transform']

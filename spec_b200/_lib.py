@@ -86,7 +86,19 @@ _PROTOS = {
     'specb200_eval_workspace_bytes': (C.c_int64, [C.c_void_p, C.c_int32]),
     'specb200_eval_forward': (C.c_int, [C.c_void_p, C.c_int32, C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_int64, C.c_int32,
                                         C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
+    'specb200_eval_create_mapped': (C.c_int, [C.POINTER(C.c_void_p), C.c_void_p, C.c_void_p, C.c_int32]),
+    'specb200_eval_forward_ex': (C.c_int, [C.c_void_p, C.c_int32, C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64,
+                                           C.c_void_p, C.c_int32, C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                           C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p]),
+    'specb200_eval_joint_errors': (C.c_int, [C.c_int32, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32,
+                                             C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     'specb200_eval_destroy': (None, [C.c_void_p]),
+    'specb200_body_create': (C.c_int, [C.POINTER(C.c_void_p), C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
+    'specb200_body_workspace_bytes': (C.c_int64, [C.c_void_p, C.c_int32]),
+    'specb200_body_forward': (C.c_int, [C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p, C.c_int64, C.c_void_p,
+                                        C.c_int64, C.c_void_p, C.c_int64, C.c_void_p]),
+    'specb200_body_regress_joints': (C.c_int, [C.c_void_p, C.c_int32, C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p]),
+    'specb200_body_destroy': (None, [C.c_void_p]),
     'specb200_preproc_create': (C.c_int, [C.POINTER(C.c_void_p), C.c_void_p, C.c_void_p]),
     'specb200_preproc_crop': (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_int64, C.c_int32, C.c_void_p, C.c_int32,
                                         C.c_double, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p]),

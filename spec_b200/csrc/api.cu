@@ -655,17 +655,70 @@ extern "C" void specb200_camtail_destroy(specb200_camtail_t* t) {
 }
 
 // =============================================================================================== HMR tail
+// SMPL constants on the device (packed by pack_smpl below)
+struct SmplConsts { float *Vt = nullptr, *Sd = nullptr, *Pd = nullptr, *Wl = nullptr, *Jt = nullptr, *Js = nullptr; };
+
 struct specb200_hmrtail {
     int C = 0, use_cam_feats = 0, use_cam = 0, ldx = 0, kin = 0;
     float focal = 5000.f, img_res = 224.f;
     float *Fx = nullptr, *c0 = nullptr, *AsT = nullptr, *init157 = nullptr;   // folded head (see tail.cu)
-    float *Vt = nullptr, *Sd = nullptr, *Pd = nullptr, *Wl = nullptr, *Jx = nullptr, *Jt = nullptr, *Js = nullptr;
+    SmplConsts smpl;
+    float* Jx = nullptr;
     int64_t last_launches = 0;
 };
 
 static bool upload(float** dst, const std::vector<float>& v) {
     if (!check_cuda(cudaMalloc(dst, v.size() * sizeof(float)), "cudaMalloc")) return false;
     return check_cuda(cudaMemcpy(*dst, v.data(), v.size() * sizeof(float), cudaMemcpyHostToDevice), "upload");
+}
+
+// SMPL constants shared by the HMR tail and the body model: validated kinematic tree, coordinate-planar repack over a padded
+// vertex axis (coalesced over vertices) and the rest-joint regression folded through the shape basis.  The integer tables
+// (c_parents is fixed; c_joint_map / c_vertex_ids belong to the HMR tail) are not touched here, so handles of any number of
+// SMPL models (neutral / male / female) coexist.
+static void free_smpl(SmplConsts& c) {
+    float* ptrs[] = {c.Vt, c.Sd, c.Pd, c.Wl, c.Jt, c.Js};
+    for (float* p : ptrs) if (p) cudaFree(p);
+    c = SmplConsts();
+}
+
+static bool check_parents(const int32_t* parents, const char* who) {
+    static const int std_parents[24] = {-1, 0, 0, 0, 1, 2, 3, 4, 5, 6, 7, 8, 9, 9, 9, 12, 13, 14, 16, 17, 18, 19, 20, 21};
+    for (int i = 0; i < 24; ++i) if (parents[i] != std_parents[i]) { set_error(std::string(who) + ": unexpected SMPL kinematic tree"); return false; }
+    return true;
+}
+
+static bool pack_smpl(SmplConsts& out, const float* v_template, const float* shapedirs, const float* posedirs, const float* J_regressor,
+                      const float* lbs_weights) {
+    const int NV = SMPL_NV, VP = SMPL_VP;
+    std::vector<float> Vt(3 * static_cast<size_t>(VP), 0.f), Sd(30 * static_cast<size_t>(VP), 0.f), Pd(207 * 3 * static_cast<size_t>(VP), 0.f),
+        Wl(24 * static_cast<size_t>(VP), 0.f);
+    for (int v = 0; v < NV; ++v) {
+        for (int c = 0; c < 3; ++c) {
+            Vt[static_cast<size_t>(c) * VP + v] = v_template[v * 3 + c];
+            for (int l = 0; l < 10; ++l) Sd[(static_cast<size_t>(l) * 3 + c) * VP + v] = shapedirs[(static_cast<size_t>(v) * 3 + c) * 10 + l];
+        }
+        for (int j = 0; j < 24; ++j) Wl[static_cast<size_t>(j) * VP + v] = lbs_weights[static_cast<size_t>(v) * 24 + j];
+    }
+    for (int k = 0; k < 207; ++k)
+        for (int v = 0; v < NV; ++v)
+            for (int c = 0; c < 3; ++c)
+                Pd[(static_cast<size_t>(k) * 3 + c) * VP + v] = posedirs[static_cast<size_t>(k) * (NV * 3) + v * 3 + c];
+    // rest-joint regression folded through the shape basis (fp64 on the host):
+    //   J = Jreg (T + S beta) = (Jreg T) + (Jreg S) beta
+    std::vector<float> Jt(72), Js(720);
+    for (int j = 0; j < 24; ++j)
+        for (int c = 0; c < 3; ++c) {
+            double a = 0.0;
+            for (int v = 0; v < NV; ++v) a += static_cast<double>(J_regressor[static_cast<size_t>(j) * NV + v]) * v_template[v * 3 + c];
+            Jt[j * 3 + c] = static_cast<float>(a);
+            for (int l = 0; l < 10; ++l) {
+                double s = 0.0;
+                for (int v = 0; v < NV; ++v) s += static_cast<double>(J_regressor[static_cast<size_t>(j) * NV + v]) * shapedirs[(static_cast<size_t>(v) * 3 + c) * 10 + l];
+                Js[(j * 3 + c) * 10 + l] = static_cast<float>(s);
+            }
+        }
+    return upload(&out.Vt, Vt) && upload(&out.Sd, Sd) && upload(&out.Pd, Pd) && upload(&out.Wl, Wl) && upload(&out.Jt, Jt) && upload(&out.Js, Js);
 }
 
 extern "C" int specb200_hmrtail_create(specb200_hmrtail_t** out, const specb200_hmr_params_t* p) {
@@ -675,8 +728,7 @@ extern "C" int specb200_hmrtail_create(specb200_hmrtail_t** out, const specb200_
                           p->posedirs, p->J_regressor, p->lbs_weights, p->J_regressor_extra};
     for (const float* q : req) if (!q) { set_error("hmrtail_create: null parameter pointer"); return 1; }
     if (!p->parents || !p->joint_map || !p->vertex_ids) { set_error("hmrtail_create: null index table"); return 1; }
-    static const int std_parents[24] = {-1, 0, 0, 0, 1, 2, 3, 4, 5, 6, 7, 8, 9, 9, 9, 12, 13, 14, 16, 17, 18, 19, 20, 21};
-    for (int i = 0; i < 24; ++i) if (p->parents[i] != std_parents[i]) { set_error("hmrtail_create: unexpected SMPL kinematic tree"); return 1; }
+    if (!check_parents(p->parents, "hmrtail_create")) return 1;
     for (int i = 0; i < 49; ++i) if (p->joint_map[i] < 0 || p->joint_map[i] >= 54) { set_error("hmrtail_create: joint_map out of range"); return 1; }
     for (int i = 0; i < 21; ++i) if (p->vertex_ids[i] < 0 || p->vertex_ids[i] >= SMPL_NV) { set_error("hmrtail_create: vertex id out of range"); return 1; }
     if ((p->in_features % 4) != 0) { set_error("hmrtail_create: in_features must be a multiple of 4"); return 1; }
@@ -725,37 +777,12 @@ extern "C" int specb200_hmrtail_create(specb200_hmrtail_t** out, const specb200_
         memcpy(&init[0], p->init_pose, sizeof(float) * 144); memcpy(&init[144], p->init_shape, sizeof(float) * 10); memcpy(&init[154], p->init_cam, sizeof(float) * 3);
         ok = ok && upload(&t->Fx, Fx) && upload(&t->c0, c0) && upload(&t->AsT, AsT) && upload(&t->init157, init);
     }
-    {   // SMPL constants, repacked coordinate-planar over a padded vertex axis (coalesced over vertices)
-        std::vector<float> Vt(3 * static_cast<size_t>(VP), 0.f), Sd(30 * static_cast<size_t>(VP), 0.f), Pd(207 * 3 * static_cast<size_t>(VP), 0.f),
-            Wl(24 * static_cast<size_t>(VP), 0.f), Jx(9 * static_cast<size_t>(VP), 0.f);
-        for (int v = 0; v < NV; ++v) {
-            for (int c = 0; c < 3; ++c) {
-                Vt[static_cast<size_t>(c) * VP + v] = p->v_template[v * 3 + c];
-                for (int l = 0; l < 10; ++l) Sd[(static_cast<size_t>(l) * 3 + c) * VP + v] = p->shapedirs[(static_cast<size_t>(v) * 3 + c) * 10 + l];
-            }
-            for (int j = 0; j < 24; ++j) Wl[static_cast<size_t>(j) * VP + v] = p->lbs_weights[static_cast<size_t>(v) * 24 + j];
+    {   // SMPL constants (shared packing) + the 9 extra-joint regressor rows, coordinate-planar like the rest
+        ok = ok && pack_smpl(t->smpl, p->v_template, p->shapedirs, p->posedirs, p->J_regressor, p->lbs_weights);
+        std::vector<float> Jx(9 * static_cast<size_t>(VP), 0.f);
+        for (int v = 0; v < NV; ++v)
             for (int q = 0; q < 9; ++q) Jx[static_cast<size_t>(q) * VP + v] = p->J_regressor_extra[static_cast<size_t>(q) * NV + v];
-        }
-        for (int k = 0; k < 207; ++k)
-            for (int v = 0; v < NV; ++v)
-                for (int c = 0; c < 3; ++c)
-                    Pd[(static_cast<size_t>(k) * 3 + c) * VP + v] = p->posedirs[static_cast<size_t>(k) * (NV * 3) + v * 3 + c];
-        // rest-joint regression folded through the shape basis (fp64 on the host):
-        //   J = Jreg (T + S beta) = (Jreg T) + (Jreg S) beta
-        std::vector<float> Jt(72), Js(720);
-        for (int j = 0; j < 24; ++j)
-            for (int c = 0; c < 3; ++c) {
-                double a = 0.0;
-                for (int v = 0; v < NV; ++v) a += static_cast<double>(p->J_regressor[static_cast<size_t>(j) * NV + v]) * p->v_template[v * 3 + c];
-                Jt[j * 3 + c] = static_cast<float>(a);
-                for (int l = 0; l < 10; ++l) {
-                    double s = 0.0;
-                    for (int v = 0; v < NV; ++v) s += static_cast<double>(p->J_regressor[static_cast<size_t>(j) * NV + v]) * p->shapedirs[(static_cast<size_t>(v) * 3 + c) * 10 + l];
-                    Js[(j * 3 + c) * 10 + l] = static_cast<float>(s);
-                }
-            }
-        ok = ok && upload(&t->Vt, Vt) && upload(&t->Sd, Sd) && upload(&t->Pd, Pd) && upload(&t->Wl, Wl) && upload(&t->Jx, Jx) &&
-             upload(&t->Jt, Jt) && upload(&t->Js, Js);
+        ok = ok && upload(&t->Jx, Jx);
     }
     ok = ok && tail_upload_tables(p->joint_map, p->vertex_ids);
     if (!ok) { specb200_hmrtail_destroy(t); return 1; }
@@ -808,9 +835,9 @@ extern "C" int specb200_hmrtail_forward(specb200_hmrtail_t* t, int32_t B, void* 
     int ks_used = HEAD_KSPLIT;                                // e.g. C = 100 yields 7 slices, not 8: sum what was written
     if (!linear_f32_launch(w.X, ldx, t->Fx, C, t->c0, nullptr, 0, w.G, 160, B, 157, C, s, HEAD_KSPLIT, static_cast<size_t>(B) * 160, &ks_used)) return 1; ++n;
     if (!head_iter_launch(w.X, ldx, C, w.G, ks_used, t->AsT, t->init157, cam_rotmat, cam_intr, img_h, t->use_cam_feats, B, s)) return 1; ++n;
-    if (!smpl_prep_launch(w.X, ldx, C, t->Jt, t->Js, w.pf, w.A, w.Jp, o->pred_pose, o->ld_pose, o->pred_pose_6d, o->ld_pose_6d,
+    if (!smpl_prep_launch(w.X, ldx, C, t->smpl.Jt, t->smpl.Js, w.pf, w.A, w.Jp, o->pred_pose, o->ld_pose, o->pred_pose_6d, o->ld_pose_6d,
                           o->pred_shape, o->ld_shape, o->pred_cam, o->ld_cam, B, s)) return 1; ++n;
-    if (!smpl_verts_launch(t->Vt, t->Sd, t->Pd, t->Wl, w.X, ldx, C, w.pf, w.A, o->smpl_vertices, o->ld_vertices, B, s)) return 1; ++n;
+    if (!smpl_verts_launch(t->smpl.Vt, t->smpl.Sd, t->smpl.Pd, t->smpl.Wl, w.X, ldx, C, w.pf, w.A, o->smpl_vertices, o->ld_vertices, B, s)) return 1; ++n;
     if (!smpl_joints_launch(o->smpl_vertices, o->ld_vertices, w.Jp, t->Jx, w.ej, w.X, ldx, C, cam_rotmat, cam_intr, bbox_scale, bbox_center,
                             img_w, img_h, o->smpl_joints3d, o->ld_joints3d, o->smpl_joints2d, o->ld_joints2d, o->pred_cam_t, o->ld_cam_t,
                             t->use_cam, t->focal, t->img_res, B, s)) return 1; n += 2;      // extra-joint regression + joints/projection
@@ -822,8 +849,77 @@ extern "C" int64_t specb200_hmrtail_last_launches(specb200_hmrtail_t* t) { retur
 
 extern "C" void specb200_hmrtail_destroy(specb200_hmrtail_t* t) {
     if (!t) return;
-    float* ptrs[] = {t->Fx, t->c0, t->AsT, t->init157, t->Vt, t->Sd, t->Pd, t->Wl, t->Jx, t->Jt, t->Js};
+    float* ptrs[] = {t->Fx, t->c0, t->AsT, t->init157, t->Jx};
     for (float* p : ptrs) if (p) cudaFree(p);
+    free_smpl(t->smpl);
+    delete t;
+}
+
+// =============================================================================================== SMPL body model
+struct specb200_body {
+    SmplConsts smpl;
+    float* JT24 = nullptr;        // J_regressor transposed, [6890][24] (regress_joints)
+};
+
+extern "C" int specb200_body_create(specb200_body_t** out, const float* v_template, const float* shapedirs, const float* posedirs,
+                                    const float* J_regressor, const float* lbs_weights, const int32_t* parents) {
+    if (!out || !v_template || !shapedirs || !posedirs || !J_regressor || !lbs_weights || !parents) { set_error("body_create: bad arguments"); return 1; }
+    if (!check_parents(parents, "body_create")) return 1;
+    specb200_body* t = new specb200_body();
+    bool ok = pack_smpl(t->smpl, v_template, shapedirs, posedirs, J_regressor, lbs_weights);
+    std::vector<float> JT(static_cast<size_t>(SMPL_NV) * 24);
+    for (int j = 0; j < 24; ++j)
+        for (int v = 0; v < SMPL_NV; ++v) JT[static_cast<size_t>(v) * 24 + j] = J_regressor[static_cast<size_t>(j) * SMPL_NV + v];
+    ok = ok && upload(&t->JT24, JT);
+    if (!ok) { specb200_body_destroy(t); return 1; }
+    *out = t;
+    return 0;
+}
+
+namespace {
+struct BodyWs { float *X, *pf, *A; size_t total; };
+BodyWs body_carve(int B, void* base) {
+    BodyWs w;
+    size_t off = 0;
+    auto take = [&](size_t nfloat) { float* p = reinterpret_cast<float*>(reinterpret_cast<uint8_t*>(base) + off); off += align_up(nfloat * sizeof(float), 256); return p; };
+    w.X = take(static_cast<size_t>(B) * BODY_XLD);
+    w.pf = take(static_cast<size_t>(B) * PF_LD);
+    w.A = take(static_cast<size_t>(B) * 288);
+    w.total = off;
+    return w;
+}
+}  // namespace
+
+extern "C" int64_t specb200_body_workspace_bytes(specb200_body_t* t, int32_t batch) {
+    if (!t || batch <= 0) { set_error("body_workspace_bytes: bad arguments"); return -1; }
+    return static_cast<int64_t>(body_carve(batch, nullptr).total);
+}
+
+extern "C" int specb200_body_forward(specb200_body_t* t, int32_t B, const float* betas, const float* pose, int32_t pose_kind,
+                                     void* workspace, int64_t workspace_bytes, float* verts, int64_t ld_verts, float* joints24,
+                                     int64_t ld_joints24, void* stream) {
+    if (!t || B <= 0 || !betas || !pose || !workspace || !verts || !joints24) { set_error("body_forward: bad arguments"); return 1; }
+    if (pose_kind != 0 && pose_kind != 1) { set_error("body_forward: pose_kind must be 0 (axis-angle) or 1 (rotation matrices)"); return 1; }
+    if ((reinterpret_cast<size_t>(workspace) & 255) != 0) { set_error("body_forward: workspace must be 256-byte aligned"); return 1; }
+    if (workspace_bytes < specb200_body_workspace_bytes(t, B)) { set_error("body_forward: workspace too small"); return 1; }
+    if (ld_verts < SMPL_NV * 3 || ld_joints24 < 72) { set_error("body_forward: output strides too small"); return 1; }
+    cudaStream_t s = static_cast<cudaStream_t>(stream);
+    NvtxRange nvtx_body("specb200:body_model (rodrigues, SMPL LBS)");
+    const BodyWs w = body_carve(B, workspace);
+    if (!body_prep_launch(betas, pose, pose_kind, t->smpl.Jt, t->smpl.Js, w.X, w.pf, w.A, joints24, ld_joints24, B, s)) return 1;
+    return smpl_verts_launch(t->smpl.Vt, t->smpl.Sd, t->smpl.Pd, t->smpl.Wl, w.X, BODY_XLD, 0, w.pf, w.A, verts, ld_verts, B, s) ? 0 : 1;
+}
+
+extern "C" int specb200_body_regress_joints(specb200_body_t* t, int32_t B, const float* verts, int64_t ld_verts, const float* rot,
+                                            float* joints24, void* stream) {
+    if (!t || B <= 0 || !verts || !joints24 || ld_verts < SMPL_NV * 3) { set_error("body_regress_joints: bad arguments"); return 1; }
+    return regress_joints24_launch(t->JT24, B, verts, ld_verts, rot, joints24, static_cast<cudaStream_t>(stream)) ? 0 : 1;
+}
+
+extern "C" void specb200_body_destroy(specb200_body_t* t) {
+    if (!t) return;
+    free_smpl(t->smpl);
+    if (t->JT24) cudaFree(t->JT24);
     delete t;
 }
 
@@ -834,38 +930,61 @@ extern "C" int specb200_linear_f32(const float* a, int32_t lda, const float* w, 
 }
 
 // =============================================================================================== eval metrics
-struct specb200_eval { float* JT = nullptr; int* map14 = nullptr; };
+struct specb200_eval { float* JT = nullptr; int* map = nullptr; int n_map = 14; };
 
-extern "C" int specb200_eval_create(specb200_eval_t** out, const float* J_host, const int32_t* map_host) {
+extern "C" int specb200_eval_create_mapped(specb200_eval_t** out, const float* J_host, const int32_t* map_host, int32_t n_map) {
     if (!out || !J_host || !map_host) { set_error("eval_create: bad arguments"); return 1; }
-    for (int i = 0; i < 14; ++i) if (map_host[i] < 0 || map_host[i] >= 17) { set_error("eval_create: joint mapper out of range"); return 1; }
+    if (n_map != 14 && n_map != 17) { set_error("eval_create: the joint mapper must have 14 or 17 entries"); return 1; }
+    for (int i = 0; i < n_map; ++i) if (map_host[i] < 0 || map_host[i] >= 17) { set_error("eval_create: joint mapper out of range"); return 1; }
     specb200_eval* t = new specb200_eval();
+    t->n_map = n_map;
     std::vector<float> JT(static_cast<size_t>(SMPL_NV) * 20, 0.f);
     for (int j = 0; j < 17; ++j)
         for (int v = 0; v < SMPL_NV; ++v) JT[static_cast<size_t>(v) * 20 + j] = J_host[static_cast<size_t>(j) * SMPL_NV + v];
     bool ok = upload(&t->JT, JT);
-    ok = ok && check_cuda(cudaMalloc(&t->map14, 14 * sizeof(int)), "cudaMalloc") &&
-         check_cuda(cudaMemcpy(t->map14, map_host, 14 * sizeof(int), cudaMemcpyHostToDevice), "upload");
+    ok = ok && check_cuda(cudaMalloc(&t->map, n_map * sizeof(int)), "cudaMalloc") &&
+         check_cuda(cudaMemcpy(t->map, map_host, n_map * sizeof(int), cudaMemcpyHostToDevice), "upload");
     if (!ok) { specb200_eval_destroy(t); return 1; }
     *out = t;
     return 0;
+}
+extern "C" int specb200_eval_create(specb200_eval_t** out, const float* J_host, const int32_t* map_host) {
+    return specb200_eval_create_mapped(out, J_host, map_host, 14);
 }
 extern "C" int64_t specb200_eval_workspace_bytes(specb200_eval_t* t, int32_t batch) {
     if (!t || batch <= 0) { set_error("eval_workspace_bytes: bad arguments"); return -1; }
     return static_cast<int64_t>(sizeof(float)) * (static_cast<int64_t>(2) * batch * 51 + static_cast<int64_t>(2) * batch * 3) + 256;
 }
+extern "C" int specb200_eval_forward_ex(specb200_eval_t* t, int32_t B, const float* pred_verts, int64_t ld_pred, const float* pred_rot,
+                                        const float* gt_kp, const float* gt_verts, int64_t ld_gt, const float* gt_rot, int32_t center_v2v,
+                                        void* ws, int64_t ws_bytes, float* mpjpe, float* pampjpe, float* v2v, float* pred_kp,
+                                        float* mpjpe_pj, float* pampjpe_pj, int32_t n_map, void* stream) {
+    if (!t || B <= 0 || !pred_verts || !ws || !mpjpe || !pampjpe) { set_error("eval_forward: bad arguments"); return 1; }
+    if (n_map != t->n_map) {
+        set_error("eval_forward: the handle evaluates " + std::to_string(t->n_map) + " joints, the caller passed " + std::to_string(n_map));
+        return 1;
+    }
+    if (ws_bytes < specb200_eval_workspace_bytes(t, B)) { set_error("eval_forward: workspace too small"); return 1; }
+    float* w = reinterpret_cast<float*>(align_up(reinterpret_cast<size_t>(ws), 16));
+    return eval_launch(t->JT, t->map, t->n_map, B, pred_verts, ld_pred, pred_rot, gt_kp, gt_verts, ld_gt, gt_rot, center_v2v, w, mpjpe,
+                       pampjpe, v2v, pred_kp, mpjpe_pj, pampjpe_pj, static_cast<cudaStream_t>(stream)) ? 0 : 1;
+}
 extern "C" int specb200_eval_forward(specb200_eval_t* t, int32_t B, const float* pred_verts, int64_t ld_pred, const float* gt_kp14,
                                      const float* gt_verts, int64_t ld_gt, int32_t center_v2v, void* ws, int64_t ws_bytes,
                                      float* mpjpe, float* pampjpe, float* v2v, float* pred_kp14, void* stream) {
-    if (!t || B <= 0 || !pred_verts || !ws || !mpjpe || !pampjpe) { set_error("eval_forward: bad arguments"); return 1; }
-    if (ws_bytes < specb200_eval_workspace_bytes(t, B)) { set_error("eval_forward: workspace too small"); return 1; }
-    float* w = reinterpret_cast<float*>(align_up(reinterpret_cast<size_t>(ws), 16));
-    return eval_launch(t->JT, t->map14, B, pred_verts, ld_pred, gt_kp14, gt_verts, ld_gt, center_v2v, w, mpjpe, pampjpe, v2v, pred_kp14,
-                       static_cast<cudaStream_t>(stream)) ? 0 : 1;
+    return specb200_eval_forward_ex(t, B, pred_verts, ld_pred, nullptr, gt_kp14, gt_verts, ld_gt, nullptr, center_v2v, ws, ws_bytes,
+                                    mpjpe, pampjpe, v2v, pred_kp14, nullptr, nullptr, 14, stream);
+}
+extern "C" int specb200_eval_joint_errors(int32_t B, int32_t n, const float* pred, const float* gt, const float* rot_pred,
+                                          const float* rot_gt, int32_t center, float* mpjpe, float* pampjpe, float* mpjpe_pj,
+                                          float* pampjpe_pj, void* stream) {
+    if (B <= 0 || !pred || !gt || !mpjpe || !pampjpe) { set_error("eval_joint_errors: bad arguments"); return 1; }
+    return joint_errors_launch(n, B, pred, gt, rot_pred, rot_gt, center, mpjpe, pampjpe, mpjpe_pj, pampjpe_pj,
+                               static_cast<cudaStream_t>(stream)) ? 0 : 1;
 }
 extern "C" void specb200_eval_destroy(specb200_eval_t* t) {
     if (!t) return;
     if (t->JT) cudaFree(t->JT);
-    if (t->map14) cudaFree(t->map14);
+    if (t->map) cudaFree(t->map);
     delete t;
 }

@@ -122,9 +122,15 @@ bool linear_f32_launch(const float* A, int lda, const float* W, int ldw, const f
                        size_t split_stride = 0, int* ksplit_used = nullptr, const LinearRedWs* red = nullptr);
 
 // eval-side metrics (eval.cu)
-bool eval_launch(const float* JT, const int* map14, int B, const float* pred_verts, long long ld_pred, const float* gt_kp14,
-                 const float* gt_verts, long long ld_gt, int center_v2v, float* ws, float* mpjpe, float* pampjpe, float* v2v,
-                 float* pred_kp14, cudaStream_t s);
+// n_map = 14 or 17 entries of `map` (into the 17 H36M joints); pred_rot / gt_rot: optional [B][9] rotations of the meshes.
+bool eval_launch(const float* JT, const int* map, int n_map, int B, const float* pred_verts, long long ld_pred, const float* pred_rot,
+                 const float* gt_kp, const float* gt_verts, long long ld_gt, const float* gt_rot, int center_v2v, float* ws,
+                 float* mpjpe, float* pampjpe, float* v2v, float* pred_kp, float* mpjpe_pj, float* pampjpe_pj, cudaStream_t s);
+// MPJPE / PA-MPJPE of already-regressed joints [B][n][3] (n = 14, 17 or 24); center = subtract joint 0 on both sides
+bool joint_errors_launch(int n, int B, const float* pred, const float* gt, const float* rot_pred, const float* rot_gt, int center,
+                         float* mpjpe, float* pampjpe, float* mpjpe_pj, float* pampjpe_pj, cudaStream_t s);
+// out [B][24][3] = rot . (J_regressor . verts); JT24 is the SMPL J_regressor transposed, [6890][24]; rot may be null
+bool regress_joints24_launch(const float* JT24, int B, const float* verts, long long ld, const float* rot, float* out, cudaStream_t s);
 
 // elementwise / layout kernels (elementwise.cu)
 bool images_to_nhwc_launch(const float* img_nchw, void* out_nhwc, int N, int H, int W, int cpad, int prec, cudaStream_t s);

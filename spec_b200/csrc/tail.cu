@@ -147,6 +147,45 @@ bool head_iter_launch(float* X, int ldx, int C, const float* G, int gsplit, cons
     return check_cuda(cudaGetLastError(), "head_iter");
 }
 
+// ------------------------------------------------------------------ SMPL kinematic chain (shared by both prep kernels)
+// One warp per image.  In: sR = the 24 joint rotations, sJ = the 24 rest joints.  Out: A[24][12] = the skinning transforms
+// G - G.[J;0] (rows of the 3x4 top) and Jposed[24][3] = the posed joints (the translation column of G).
+__device__ __forceinline__ void smpl_chain(const float (*sR)[9], const float (*sJ)[3], float (*sG)[12], float* __restrict__ A_out,
+                                           float* __restrict__ Jposed, int lane)
+{
+    // kinematic chain: G_0 = [R_0 | J_0];  G_i = G_par * [R_i | J_i - J_par]
+    if (lane < 9) sG[0][(lane / 3) * 4 + (lane % 3)] = sR[0][lane];
+    else if (lane < 12) sG[0][(lane - 9) * 4 + 3] = sJ[0][lane - 9];
+    __syncwarp();
+    for (int i = 1; i < 24; ++i) {
+        const int par = c_parents[i];
+        float v = 0.f;
+        if (lane < 9) {
+            const int r = lane / 3, c = lane % 3;
+            v = sG[par][r * 4 + 0] * sR[i][0 * 3 + c] + sG[par][r * 4 + 1] * sR[i][1 * 3 + c] + sG[par][r * 4 + 2] * sR[i][2 * 3 + c];
+        } else if (lane < 12) {
+            const int r = lane - 9;
+            const float rx = sJ[i][0] - sJ[par][0], ry = sJ[i][1] - sJ[par][1], rz = sJ[i][2] - sJ[par][2];
+            v = sG[par][r * 4 + 0] * rx + sG[par][r * 4 + 1] * ry + sG[par][r * 4 + 2] * rz + sG[par][r * 4 + 3];
+        }
+        __syncwarp();
+        if (lane < 9) sG[i][(lane / 3) * 4 + (lane % 3)] = v;
+        else if (lane < 12) sG[i][(lane - 9) * 4 + 3] = v;
+        __syncwarp();
+    }
+    if (lane < 24) {
+        const float* G = sG[lane];
+        float* A = A_out + lane * 12;
+        const float jx = sJ[lane][0], jy = sJ[lane][1], jz = sJ[lane][2];
+#pragma unroll
+        for (int r = 0; r < 3; ++r) {
+            A[r * 4 + 0] = G[r * 4 + 0]; A[r * 4 + 1] = G[r * 4 + 1]; A[r * 4 + 2] = G[r * 4 + 2];
+            A[r * 4 + 3] = G[r * 4 + 3] - (G[r * 4 + 0] * jx + G[r * 4 + 1] * jy + G[r * 4 + 2] * jz);
+            Jposed[lane * 3 + r] = G[r * 4 + 3];
+        }
+    }
+}
+
 // ------------------------------------------------------------------ SMPL prep: rot6d, rest joints, kinematic chain
 // grid = B, block = 32.
 __global__ void __launch_bounds__(32)
@@ -202,37 +241,7 @@ smpl_prep_kernel(const float* __restrict__ X, int ldx, int C, const float* __res
     }
     if (lane == 0) pf[static_cast<size_t>(b) * PF_LD + 207] = 0.f;   // K padding column
     __syncwarp();
-    // kinematic chain: G_0 = [R_0 | J_0];  G_i = G_par * [R_i | J_i - J_par]
-    if (lane < 9) sG[0][(lane / 3) * 4 + (lane % 3)] = sR[0][lane];
-    else if (lane < 12) sG[0][(lane - 9) * 4 + 3] = sJ[0][lane - 9];
-    __syncwarp();
-    for (int i = 1; i < 24; ++i) {
-        const int par = c_parents[i];
-        float v = 0.f;
-        if (lane < 9) {
-            const int r = lane / 3, c = lane % 3;
-            v = sG[par][r * 4 + 0] * sR[i][0 * 3 + c] + sG[par][r * 4 + 1] * sR[i][1 * 3 + c] + sG[par][r * 4 + 2] * sR[i][2 * 3 + c];
-        } else if (lane < 12) {
-            const int r = lane - 9;
-            const float rx = sJ[i][0] - sJ[par][0], ry = sJ[i][1] - sJ[par][1], rz = sJ[i][2] - sJ[par][2];
-            v = sG[par][r * 4 + 0] * rx + sG[par][r * 4 + 1] * ry + sG[par][r * 4 + 2] * rz + sG[par][r * 4 + 3];
-        }
-        __syncwarp();
-        if (lane < 9) sG[i][(lane / 3) * 4 + (lane % 3)] = v;
-        else if (lane < 12) sG[i][(lane - 9) * 4 + 3] = v;
-        __syncwarp();
-    }
-    if (lane < 24) {
-        const float* G = sG[lane];
-        float* A = Amat + (static_cast<size_t>(b) * 24 + lane) * 12;
-        const float jx = sJ[lane][0], jy = sJ[lane][1], jz = sJ[lane][2];
-#pragma unroll
-        for (int r = 0; r < 3; ++r) {
-            A[r * 4 + 0] = G[r * 4 + 0]; A[r * 4 + 1] = G[r * 4 + 1]; A[r * 4 + 2] = G[r * 4 + 2];
-            A[r * 4 + 3] = G[r * 4 + 3] - (G[r * 4 + 0] * jx + G[r * 4 + 1] * jy + G[r * 4 + 2] * jz);
-            Jposed[(static_cast<size_t>(b) * 24 + lane) * 3 + r] = G[r * 4 + 3];
-        }
-    }
+    smpl_chain(sR, sJ, sG, Amat + static_cast<size_t>(b) * 288, Jposed + static_cast<size_t>(b) * 72, lane);
 }
 
 bool smpl_prep_launch(const float* X, int ldx, int C, const float* Jt, const float* Js, float* pf, float* Amat,
@@ -241,6 +250,70 @@ bool smpl_prep_launch(const float* X, int ldx, int C, const float* Jt, const flo
     smpl_prep_kernel<<<B, 32, 0, s>>>(X, ldx, C, Jt, Js, pf, Amat, Jposed, o_pose, ld_pose, o_pose6d, ld_pose6d,
                                       o_shape, ld_shape, o_cam, ld_cam, B);
     return check_cuda(cudaGetLastError(), "smpl_prep");
+}
+
+// ------------------------------------------------------------------ body-model prep: axis-angle / rotation matrices + betas
+// The smplx SMPL forward (lbs with pose2rot) from caller-given parameters, for the evaluation side (BodyModel).  grid = B,
+// block = 32.  pose_kind 0: pose = axis-angle [B][72], turned into rotations with smplx's batch_rodrigues
+//     angle = |r + 1e-8|,  k = r / angle,  R = I + sin(angle) K + (1 - cos(angle)) K^2   (K = [k]_x);
+// pose_kind 1: pose = rotation matrices [B][24][9], copied (pose2rot=False).  The betas are staged in the X row buffer
+// ([B][BODY_XLD], read by smpl_verts_kernel at column 144 with C = 0); the posed joints go to joints[b * ld_joints].
+__global__ void __launch_bounds__(32)
+body_prep_kernel(const float* __restrict__ betas, const float* __restrict__ pose, int pose_kind, const float* __restrict__ Jt,
+                 const float* __restrict__ Js, float* __restrict__ X, float* __restrict__ pf, float* __restrict__ Amat,
+                 float* __restrict__ joints, long long ld_joints, int B)
+{
+    __shared__ float sR[24][9];
+    __shared__ float sJ[24][3];
+    __shared__ float sG[24][12];
+    __shared__ float sBeta[10];
+    const int b = blockIdx.x, lane = threadIdx.x;
+    if (lane < 10) {
+        const float be = betas[b * 10 + lane];
+        sBeta[lane] = be;
+        X[static_cast<size_t>(b) * BODY_XLD + 144 + lane] = be;
+    }
+    __syncwarp();
+    if (lane < 24) {
+        float* R = sR[lane];
+        if (pose_kind == 0) {
+            const float* r = pose + static_cast<size_t>(b) * 72 + lane * 3;
+            const float ax = r[0] + 1e-8f, ay = r[1] + 1e-8f, az = r[2] + 1e-8f;
+            const float angle = sqrtf(ax * ax + ay * ay + az * az);
+            const float kx = r[0] / angle, ky = r[1] / angle, kz = r[2] / angle;
+            const float sn = sinf(angle), omc = 1.f - cosf(angle);
+            // K = [[0,-kz,ky],[kz,0,-kx],[-ky,kx,0]];  K^2 = k k^T - |k|^2 I
+            R[0] = 1.f + omc * (-kz * kz - ky * ky); R[1] = -sn * kz + omc * (ky * kx);        R[2] = sn * ky + omc * (kz * kx);
+            R[3] = sn * kz + omc * (kx * ky);        R[4] = 1.f + omc * (-kz * kz - kx * kx); R[5] = -sn * kx + omc * (kz * ky);
+            R[6] = -sn * ky + omc * (kx * kz);       R[7] = sn * kx + omc * (ky * kz);        R[8] = 1.f + omc * (-ky * ky - kx * kx);
+        } else {
+            const float* m = pose + (static_cast<size_t>(b) * 24 + lane) * 9;
+#pragma unroll
+            for (int e = 0; e < 9; ++e) R[e] = m[e];
+        }
+        if (lane >= 1) {
+            float* p = pf + static_cast<size_t>(b) * PF_LD + (lane - 1) * 9;
+#pragma unroll
+            for (int e = 0; e < 9; ++e) p[e] = R[e] - ((e == 0 || e == 4 || e == 8) ? 1.f : 0.f);
+        }
+        // rest joints J = Jt + Js . beta (as smpl_prep_kernel)
+#pragma unroll
+        for (int c = 0; c < 3; ++c) {
+            float acc = Jt[lane * 3 + c];
+#pragma unroll
+            for (int l = 0; l < 10; ++l) acc = fmaf(Js[(lane * 3 + c) * 10 + l], sBeta[l], acc);
+            sJ[lane][c] = acc;
+        }
+    }
+    if (lane == 0) pf[static_cast<size_t>(b) * PF_LD + 207] = 0.f;   // K padding column
+    __syncwarp();
+    smpl_chain(sR, sJ, sG, Amat + static_cast<size_t>(b) * 288, joints + b * ld_joints, lane);
+}
+
+bool body_prep_launch(const float* betas, const float* pose, int pose_kind, const float* Jt, const float* Js, float* X, float* pf,
+                      float* Amat, float* joints, long long ld_joints, int B, cudaStream_t s) {
+    body_prep_kernel<<<B, 32, 0, s>>>(betas, pose, pose_kind, Jt, Js, X, pf, Amat, joints, ld_joints, B);
+    return check_cuda(cudaGetLastError(), "body_prep");
 }
 
 // ------------------------------------------------------------------ SMPL vertices

@@ -55,28 +55,34 @@ def _read_smpl_file(path):
                            '(see spec_b200/hmr.py::_read_smpl_file)') from e
 
 
-def _load_smpl_data():
+def _load_smpl_data(gender='neutral', need_extra=True):
     """SMPL constants from ``SMPL_NEUTRAL.npz`` / ``SMPL_NEUTRAL.pkl`` under SMPL_MODEL_DIR (spec/config.py:35) plus
-    ``J_regressor_extra.npy`` (config.py:36)."""
-    cands = [os.path.join(SMPL_MODEL_DIR, n) for n in ('SMPL_NEUTRAL.npz', 'SMPL_NEUTRAL.pkl')]
+    ``J_regressor_extra.npy`` (config.py:36).  ``gender`` picks ``SMPL_{NEUTRAL,MALE,FEMALE}``; ``need_extra=False`` (the
+    body model, which has no extra joints) does without ``J_regressor_extra.npy``."""
+    if gender not in ('neutral', 'male', 'female'):
+        raise ValueError(f"gender must be 'neutral', 'male' or 'female', got {gender!r}")
+    stem = 'SMPL_' + gender.upper()
+    cands = [os.path.join(SMPL_MODEL_DIR, stem + ext) for ext in ('.npz', '.pkl')]
     path = next((c for c in cands if os.path.exists(c)), None)
-    if path is not None and os.path.exists(JOINT_REGRESSOR_TRAIN_EXTRA):
+    if path is not None and (not need_extra or os.path.exists(JOINT_REGRESSOR_TRAIN_EXTRA)):
         d = _read_smpl_file(path)
         out = {k: _dense(d[k]).astype(np.float32) for k in ('v_template', 'shapedirs', 'J_regressor')}
         out['shapedirs'] = out['shapedirs'][:, :, :10]
         pd = _dense(d['posedirs']).astype(np.float32)
         out['posedirs'] = pd.reshape(-1, pd.shape[-1]).T if pd.ndim == 3 else pd
         out['lbs_weights'] = _dense(d['weights'] if 'weights' in d else d['lbs_weights']).astype(np.float32)
-        out['J_regressor_extra'] = np.load(JOINT_REGRESSOR_TRAIN_EXTRA).astype(np.float32)
+        if need_extra:
+            out['J_regressor_extra'] = np.load(JOINT_REGRESSOR_TRAIN_EXTRA).astype(np.float32)
         out['parents'] = np.asarray(SMPL_PARENTS, dtype=np.int64)
         return out
     if not synthetic_assets_allowed():
         raise FileNotFoundError(
-            f'SMPL model not found: looked for {cands} and {JOINT_REGRESSOR_TRAIN_EXTRA!r} (set SPECB200_SMPL_DIR / '
-            'SPECB200_J_REGRESSOR_EXTRA, pass smpl_data=, or opt in to seeded synthetic constants with SPECB200_SYNTHETIC_ASSETS=1)')
+            f'SMPL model not found: looked for {cands}' + (f' and {JOINT_REGRESSOR_TRAIN_EXTRA!r}' if need_extra else '') +
+            ' (set SPECB200_SMPL_DIR / SPECB200_J_REGRESSOR_EXTRA, pass smpl_data=, or opt in to seeded synthetic constants with '
+            'SPECB200_SYNTHETIC_ASSETS=1)')
     warnings.warn(f'SMPL model not found under {SMPL_MODEL_DIR!r}: using seeded SYNTHETIC SMPL constants '
                   '(right shapes, meaningless geometry; SPECB200_SYNTHETIC_ASSETS=1)', stacklevel=3)
-    return synthetic_smpl_data(0)
+    return synthetic_smpl_data(('neutral', 'male', 'female').index(gender))
 
 
 def _load_mean_params():
